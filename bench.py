@@ -2,6 +2,7 @@
 """Benchmark of the I-ADMM-LSTM unrolled solve path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu] [--workload W] [--gate-mode M] [--batch B]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (`--workload`; the default `solve` is the headline BASELINE config 2, the line the driver records):
@@ -27,6 +28,7 @@ baseline/_ref (kind "reference") when that copy travelled with the snapshot, els
 device-timed): the like-for-like "what torch gives you on this GPU" number, also reported as `gpu_reference` in our line.
 """
 import argparse
+import dataclasses
 import json
 import os
 import statistics
@@ -100,7 +102,14 @@ def parse_args():
                                                                   "iadmm_allreduce_grads (raw NCCL communicator) instead of torch.distributed")
     ap.add_argument("--graph", action="store_true", help="train: capture scale_data + the window (forward, loss, backward) in ONE CUDA graph "
                                                           "and replay it per step (the library only enqueues on the caller's stream)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (rank 0's instances; "
+                         "at most 64 MB in all, larger outputs as a fixed seeded sample of their rows, see dump_outputs; implies --no-balance)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if a.workload == "config5":
         a.nvar = 5000
     if a.workload == "hidden200":
@@ -117,6 +126,41 @@ def device_qp_batch(B, n, mi, me, seed, dev):
     from iadmm_b200.data import generate_qp_batch
     d = generate_qp_batch(B, n, mi, me, seed, dev)
     return d["Q"], d["p"], d["A0"], d["zl"], d["zu"]
+
+
+# ---------------------------------------------------------------------------------------------------
+# --dump-outputs: the arrays of the last timed step, for comparing two builds output for output
+# ---------------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 * 10**6
+NPY_HEADER = 256          # bytes reserved per .npy file for its header
+
+
+def dump_outputs(outdir, arrays):
+    """Write each tensor of `arrays` (name -> tensor) as outdir/<name>.npy, float64 if it is float64 else float32, within
+    DUMP_BYTES in all.  Smallest first, each array gets an equal share of what the ones before it left; an array larger than
+    its share is viewed as rows of its last dimension and stored as a sample of them, drawn by a generator with a fixed seed,
+    so every run and every build at the same shape picks the same rows.  Their indices go to <name>_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    items = sorted(((k, v.detach()) for k, v in arrays.items() if v is not None), key=lambda kv: (kv[1].numel(), kv[0]))
+    left = DUMP_BYTES - 2 * NPY_HEADER * len(items)
+    for i, (name, t) in enumerate(items):
+        dt = torch.float64 if t.dtype == torch.float64 else torch.float32
+        esize = 8 if dt == torch.float64 else 4
+        share = left // (len(items) - i)
+        if t.numel() * esize <= share:
+            out = t.to(dt).cpu()
+        else:
+            rows = t.reshape(-1, t.shape[-1] if t.dim() > 1 else 1)
+            keep = share // (rows.shape[1] * esize + 8)
+            if keep < 1:
+                raise RuntimeError(f"--dump-outputs: one row of {name} {tuple(t.shape)} does not fit its share of {DUMP_BYTES} bytes")
+            idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            out = rows[idx.to(rows.device)].to(dt).cpu()
+            np.save(os.path.join(outdir, name + "_rows.npy"), idx.numpy().astype(np.float64))
+            left -= idx.numel() * 8
+        np.save(os.path.join(outdir, name + ".npy"), out.numpy())
+        left -= out.numel() * esize
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -264,7 +308,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     n, h = args.nvar, args.hidden
     workload = workload_name(args)
     if args.impl == "reference-gpu":
@@ -350,7 +394,7 @@ def run_ours(args):
     n_gpus = world
     B, n, mi, me, h, K = args.batch, args.nvar, args.nvar // 2, args.nvar // 2, args.hidden, args.iters
     m, N = mi + me, n + mi + me
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     L = ia.lib()
 
     torch.manual_seed(17)                                    # identical random-init weights on every rank
@@ -358,7 +402,8 @@ def run_ours(args):
     # N > 1: the job is N*B independent instances.  GPUs of one box differ by several per cent under the power cap, so after
     # the warm-up the instances are re-sharded in proportion to each GPU's measured rate (iadmm_b200.dist.balance_by_rate: one
     # all-gather of a float per rank at set-up; the solve itself has no collective).  Every rank generates some spare instances.
-    balance = world > 1 and not args.no_balance
+    # (not with --dump-outputs: rank 0's share, and so the shapes it dumps, must follow from the arguments alone)
+    balance = world > 1 and not args.no_balance and not args.dump_outputs
     B_cap = B + max(8, B // 8) if balance else B
     sparse_mode = args.workload == "sparse"
     if sparse_mode and "--sparse" not in sys.argv:
@@ -436,6 +481,8 @@ def run_ours(args):
         ia._lib.check(L.iadmm_profile_end(byref(kkt_ms), byref(gate_ms), byref(tail_ms), byref(nit)))
         clocks = sampler.stop() if sampler else None
         finite = bool(torch.isfinite(r.x).all() and torch.isfinite(r.pri).all())
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {f.name: getattr(r, f.name) for f in dataclasses.fields(r)})
 
         # ---- e2e: same step through the public API from pinned host buffers --------------------------
         e2e = None
@@ -644,7 +691,7 @@ def run_train(args):
         dist.init_process_group("nccl", device_id=dev)
     B, n, mi, me, h, TL = args.batch, args.nvar, args.nvar // 2, args.nvar // 2, args.hidden, args.tl
     m, N = mi + me, n + mi + me
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     L = ia.lib()
     torch.manual_seed(17)                                    # identical initial weights on every rank
     model = ia.LSTM(None, 2, h, TL, dev, gate_mode=args.gate_mode)
@@ -742,6 +789,12 @@ def run_train(args):
     ia._lib.check(L.iadmm_profile_end_kinds(pms, pcnt, kinds))
     clocks = sampler.stop() if sampler else None
     ar_ms = sum(a.elapsed_time(b) for a, b in ar_ev) if world > 1 else 0.0
+    if args.dump_outputs and rank == 0:
+        # the window's loss, the gradients it left in .grad and the weights after the Adam step
+        outs = {"loss": loss.reshape(-1)}
+        for name, prm in model.named_parameters():
+            outs[name], outs["grad_" + name] = prm, prm.grad
+        dump_outputs(args.dump_outputs, outs)
     loss_v = float(loss)
     mem_gb = torch.cuda.max_memory_allocated() / 1e9
 

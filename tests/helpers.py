@@ -70,3 +70,59 @@ def oracle_pair(prm, K, mi, me, qp, h, scaling_ites=10, sigma=6e-6, form="block"
         r = orc.solve({k: v.to(dt) for k, v in prm.items()}, K, mi, me, Qs, ps, As, zls, zus, sigma, h, form=form)
         out.append((r, (Qs, ps, As, zls, zus), sc))
     return out[0][0], out[1][0], out[0][1], out[0][2]
+
+
+# K=100 at the headline shape against the reference's fp32 computation on the GPU (test_gpu_production_shapes and
+# tests/golden/make_k100_config2_golden.py): inputs from the oracle's generators, seed 43
+K100_SHAPE = dict(B=16, n=1000, mi=500, me=500, h=800, K=100, seed=43)
+K100_ROWS = (137, 712)                  # sampled rows of the scaled Q and A0: one inequality, one equality row
+
+
+def k100_inputs(device):
+    from oracle import iadmm_oracle as orc
+    s = K100_SHAPE
+    qp = orc.qp_instances(s["B"], s["n"], s["mi"], s["me"], seed=s["seed"])
+    return ({k: qp[k].to(device) for k in ("Q", "p", "A0", "zl", "zu")},
+            orc.lstm_parameters(s["h"], s["K"], seed=s["seed"]))
+
+
+def k100_record(data, d, e, c, x, y, z, pri, dual):
+    """What the K=100 comparison looks at, as float32 CPU tensors: the Ruiz diagonals d [B,n], e [B,m], c [B], the scaled
+    p, zl, zu and rows K100_ROWS of the scaled Q and A0, the final x, y, z and the [K,B] residual traces."""
+    Q, p, A0, zl, zu = data
+    rows = list(K100_ROWS)
+    rec = dict(d=d, e=e, c=c.reshape(-1), p=p, zl=zl, zu=zu, Q_rows=Q[:, rows], A0_rows=A0[:, rows],
+               x=x, y=y, z=z, pri=pri, dual=dual)
+    return {k: v.detach().float().cpu().contiguous() for k, v in rec.items()}
+
+
+def k100_reference_record(device):
+    """The reference's computation of the K=100 case in stock PyTorch fp32 on `device` (TF32 off): Ruiz scaling
+    (methods/scaling.py), K calls of the cell with the dense KKT matrix (models/lstm.py:47-96), primal_dual_loss after each
+    (utils.py:68-71).  Runs the reference's own modules when baseline/_ref holds them, else the oracle's restatement of them
+    (form="dense"; test_oracle_golden pins it to outputs of the reference's modules).  Returns (k100_record, source)."""
+    from baseline import ref_arm
+    from oracle import iadmm_oracle as orc
+    torch.backends.cuda.matmul.allow_tf32 = False
+    s = K100_SHAPE
+    qp, prm = k100_inputs(device)
+    raw = [qp[k] for k in ("Q", "p", "A0", "zl", "zu")]
+    if ref_arm.available():
+        r = ref_arm.solve(ref_arm.make_model(prm, s["h"], s["K"], device), s["K"], s["mi"], s["me"], *raw, ref_arm.SIGMA, 10)
+        sc = r["scaling"]
+        d, e = (torch.diagonal(M, dim1=1, dim2=2) for M in (sc.D, sc.E))
+        rec = k100_record(r["data"], d, e, sc.c, *(r[k] for k in ("x", "y", "z", "pri", "dual")))
+        source = "the reference's modules (baseline/_ref)"
+    else:
+        default = torch.get_default_device()
+        torch.set_default_device(device)          # the oracle allocates its work tensors without naming a device
+        try:
+            Qs, ps, As, zls, zus, sc = orc.ruiz_equilibrate(*raw, 10)
+            r = orc.solve({k: v.to(device) for k, v in prm.items()}, s["K"], s["mi"], s["me"], Qs, ps, As, zls, zus, 6e-6, s["h"],
+                          form="dense")
+        finally:
+            torch.set_default_device(default)
+        rec = k100_record((Qs, ps, As, zls, zus), sc.d, sc.e, sc.c, r.x, r.y, r.z, r.pri, r.dual)
+        source = "the oracle's restatement of the reference's modules (oracle/iadmm_oracle.py, form='dense')"
+    where = torch.cuda.get_device_name(device) if torch.device(device).type == "cuda" else "CPU"
+    return rec, f"{source} on {where}, torch {torch.__version__}, fp32, TF32 off"

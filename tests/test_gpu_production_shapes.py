@@ -8,7 +8,8 @@ import sys
 import pytest
 import torch
 
-from helpers import rel_err, assert_parity, oracle_pair
+from helpers import (rel_err, assert_parity, oracle_pair, load_golden, K100_SHAPE, K100_ROWS, k100_inputs, k100_record,
+                     k100_reference_record)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -81,30 +82,37 @@ def test_production_kernel_at_production_batch_bit_exact():
 def test_k100_config2_vs_unmodified_reference_on_this_gpu():
     """The like-for-like oracle of SURVEY section 8(c/d): the reference's OWN modules (baseline/_ref, unmodified) with
     device='cuda' -- stock PyTorch fp32 kernels, TF32 off -- against the drop-in on the same GPU, same inputs, same weights:
-    K=100, n=1000, 500+500, hidden_dim=800, --scaling, 16 instances.  x^K, y^K, z^K and the residual traces within 1e-4."""
+    K=100, n=1000, 500+500, hidden_dim=800, --scaling, 16 instances.  x^K, y^K, z^K and the residual traces within 1e-4; the
+    Ruiz diagonals, the scaled p, zl, zu and two rows of the scaled Q and A0 within 1e-6.  Without the reference's modules in
+    baseline/_ref, the reference side is the stored outputs of the same computation (tests/golden/k100_config2.npz, written by
+    tests/golden/make_k100_config2_golden.py; its `source` says what produced them)."""
     sys.path.insert(0, ROOT)
     from baseline import ref_arm
-    if not ref_arm.available():
-        pytest.skip("baseline/_ref is not in this snapshot (build() copies it in the build container)")
     import iadmm_b200 as ia
-    from oracle import iadmm_oracle as orc
-    torch.backends.cuda.matmul.allow_tf32 = False
-    B, n, mi, me, h, K = 16, 1000, 500, 500, 800, 100
-    qp = {k: v.to(DEV) for k, v in orc.qp_instances(B, n, mi, me, seed=43).items()}
-    prm = orc.lstm_parameters(h, K, seed=43)
-    ref = ref_arm.solve(ref_arm.make_model(prm, h, K, DEV), K, mi, me, qp["Q"], qp["p"], qp["A0"], qp["zl"], qp["zu"], 6e-6, 10)
+    s = K100_SHAPE
+    B, n, mi, me, h, K = (s[k] for k in ("B", "n", "mi", "me", "h", "K"))
+    if ref_arm.available():
+        ref, source = k100_reference_record(DEV)
+    else:
+        g = load_golden("k100_config2")
+        assert [int(v) for v in g["meta"]] == [s[k] for k in ("B", "n", "mi", "me", "h", "K", "seed")]
+        assert tuple(int(v) for v in g["rows"]) == K100_ROWS
+        ref, source = {k: torch.from_numpy(v) for k, v in g.items() if k not in ("source", "meta", "rows")}, str(g["source"])
+    qp, prm = k100_inputs(DEV)
     sc = ia.Scaling(n, mi + me, 10, DEV)
     data = sc.scale_data(qp["Q"], qp["p"], qp["A0"], qp["zl"], qp["zu"])
-    for a, b in zip(data, ref["data"]):                          # Ruiz: the reference's O(n^3) dense-diag form on the GPU
-        assert rel_err(a, b) < 1e-6
     model = make_model(prm, h, K)
     with torch.no_grad():
         r = model.solve(K, mi, me, *data, 6e-6, scaling=sc)
     torch.cuda.synchronize()
-    errs = {k: rel_err(getattr(r, k), ref[k]) for k in ("x", "y", "z", "pri", "dual")}
+    ours = k100_record(data, sc.d, sc.e, sc.c_vec, r.x, r.y, r.z, r.pri, r.dual)
+    assert sorted(ours) == sorted(ref)
+    for k in ("d", "e", "c", "p", "zl", "zu", "Q_rows", "A0_rows"):     # Ruiz: the reference's O(n^3) dense-diag form on the GPU
+        assert rel_err(ours[k], ref[k]) < 1e-6, k
+    errs = {k: rel_err(ours[k], ref[k]) for k in ("x", "y", "z", "pri", "dual")}
     # per instance too: the worst instance, not only the batch norm
-    worst = {k: max(rel_err(getattr(r, k)[i], ref[k][i]) for i in range(B)) for k in ("x", "y", "z")}
-    print("K=100 config-2 vs reference-on-GPU", {k: f"{v:.1e}" for k, v in errs.items()}, "worst instance", {k: f"{v:.1e}" for k, v in worst.items()})
+    worst = {k: max(rel_err(ours[k][i], ref[k][i]) for i in range(B)) for k in ("x", "y", "z")}
+    print("K=100 config-2 vs", source, {k: f"{v:.1e}" for k, v in errs.items()}, "worst instance", {k: f"{v:.1e}" for k, v in worst.items()})
     for k, v in errs.items():
         assert v <= 1e-4, (k, v)
     for k, v in worst.items():
