@@ -414,13 +414,17 @@ int launch_tc_gemm_nt(const __half* A_hi, const __half* A_lo, const __half* B_hi
       (rc = mk(&mb_hi, B_hi, N, ldb, pair ? kGpBoxRows : kGmBN)) || (rc = mk(&mb_lo, B_lo, N, ldb, pair ? kGpBoxRows : kGmBN)))
     return rc;
   GemmParams P;
-  if (splits < 1 || (splits > 1 && (!part || (M * ldc) % 4 != 0))) IADMM_FAIL(IADMM_ESHAPE, "tc_gemm: bad split-K arguments");
-  P.C = (splits > 1) ? part : C; P.scale = scale; P.M = M; P.N = N; P.K = K; P.ldc = ldc;
+  if (K < 1 || splits < 1 || (splits > 1 && (!part || (M * ldc) % 4 != 0))) IADMM_FAIL(IADMM_ESHAPE, "tc_gemm: bad split-K arguments");
   P.n_tiles = (int)((N + kGmBN - 1) / kGmBN);
   P.k_blocks = (int)((K + kGmBK - 1) / kGmBK);
-  P.splits = splits;
-  P.prod_mask = prod_mask | 4;
   P.kb_per_split = (P.k_blocks + splits - 1) / splits;
+  // Only splits that cover K blocks are launched: when the factor does not divide the K blocks evenly the trailing splits
+  // can be left with none (125 blocks in 15 splits of 9 cover 14 splits), and such a work unit would store an accumulator
+  // that no MMA of this launch wrote.
+  splits = (P.k_blocks + P.kb_per_split - 1) / P.kb_per_split;
+  P.splits = splits;
+  P.C = (splits > 1) ? part : C; P.scale = scale; P.M = M; P.N = N; P.K = K; P.ldc = ldc;
+  P.prod_mask = prod_mask | 4;
   const int tile_rows = pair ? 2 * kTcBM : kTcBM;
   P.num_tiles = ((M + tile_rows - 1) / tile_rows) * P.n_tiles;
   static PerDeviceOnce attr, attr_pair;
