@@ -55,7 +55,7 @@ int launch_build_kkt(int B, int n, int m, int num_ineq, const float* Q, const fl
                      const float* x, const float* y, const float* z, const Sched* sched_t, float sigma, float* K,
                      float* rhs, float* rho_vec, cudaStream_t st);
 
-static int check_device() {
+int check_device() {
   int dev = 0, major = 0;
   IADMM_CUDA(cudaGetDevice(&dev));
   IADMM_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
@@ -71,7 +71,6 @@ struct SolveWs {
   TcState tc;             // TC: fp16 hi/lo ping-pong
   float* c_il;            // F16F8: row-interleaved cell state [h/8][rows_p][8] (see gates_tc.cu)
   long rows_p;
-  int tiles;
   size_t bytes;
 };
 
@@ -98,30 +97,24 @@ void prof_end(int kind, cudaStream_t st) {
   g_prof.open[kind] = -(g_prof.open[kind] + 2);       // closed: remembered as -(i+2)
 }
 
-static int is_tc(int mode) {
-  return mode == IADMM_GATES_TC_3XFP16 || mode == IADMM_GATES_TC_1XFP16 || mode == IADMM_GATES_TC_F16F8 || mode == IADMM_GATES_TC_F16F8U;
-}
-static int is_f16f8(int mode) { return mode == IADMM_GATES_TC_F16F8 || mode == IADMM_GATES_TC_F16F8U; }
-
-static int plan_workspace(int B, int n, int m, int num_ineq, int h, int mode, void* base, SolveWs* ws) {
-  if (mode != IADMM_GATES_SIMT_FP32 && !is_tc(mode)) IADMM_FAIL(IADMM_EMODE, "unknown gate mode %d", mode);
-  if (is_tc(mode) && (h % 8 != 0)) IADMM_FAIL(IADMM_EMODE, "tensor-core gate modes need hidden_dim %% 8 == 0 (got %d)", h);
-  // (fp16+fp8 mode: hidden_dim % 16 == 8, e.g. configs/QP.yaml's 200, runs on the row-interleaved kernels only: the last 16-unit
-  // group of the e4m3 planes is half padding)
+// The layout depends on the gate mode alone (the path and the product count of the plan), not on K or the flags: one
+// workspace serves every call of a mode, and resumed calls find the planes where the previous call left them.
+static void plan_workspace(int B, int n, int m, int num_ineq, int h, const GatePlan& gp, void* base, SolveWs* ws) {
+  const bool tc = gp.path != kGatesFp32;
   ws->d = make_kkt_dims(B, n, m, num_ineq);
   const size_t rows = (size_t)B * (n + m);
-  ws->tiles = is_tc(mode) ? tc_gate_tiles(h) : simt_gate_tiles(h);
+  const int tiles = tc ? tc_gate_tiles(h) : simt_gate_tiles(h);       // bound of the plan's head_slots
   char* p = static_cast<char*>(base);
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return base ? p + o : nullptr; };
   float* kkt = reinterpret_cast<float*>(take(kkt_scratch_floats(ws->d) * sizeof(float)));
   if (base) kkt_scratch_carve(ws->d, kkt, &ws->s);
-  ws->head_part = reinterpret_cast<float*>(take((size_t)ws->tiles * rows * sizeof(float)));
+  ws->head_part = reinterpret_cast<float*>(take((size_t)tiles * rows * sizeof(float)));
   ws->h_alt = nullptr; ws->c_il = nullptr; ws->rows_p = (long)rows;
   memset(&ws->tc, 0, sizeof(ws->tc));
-  if (is_tc(mode)) {
+  if (tc) {
     // the F16F8 solve keeps its state row-interleaved: rows padded to a multiple of 128
-    const bool il = is_f16f8(mode);
+    const bool il = gp.nprod == 2;
     ws->rows_p = il ? il_rows((long)rows) : (long)rows;
     const size_t rp = (size_t)ws->rows_p;
     const size_t hb = rp * (size_t)h * sizeof(__half);
@@ -138,7 +131,6 @@ static int plan_workspace(int B, int n, int m, int num_ineq, int h, int mode, vo
     ws->h_alt = reinterpret_cast<float*>(take(rows * (size_t)h * sizeof(float)));
   }
   ws->bytes = off;
-  return IADMM_OK;
 }
 
 }  // namespace iadmm
@@ -196,9 +188,11 @@ int iadmm_ruiz(const float* Q, const float* p, const float* A0, const float* zl,
 
 int iadmm_solve_workspace_bytes(int B, int n, int m, int h, int mode, size_t* bytes) {
   if (B <= 0 || n <= 0 || m < 0 || h <= 0 || !bytes) IADMM_FAIL(IADMM_ESHAPE, "solve_workspace_bytes: B=%d n=%d m=%d h=%d", B, n, m, h);
-  SolveWs ws;
-  int rc = plan_workspace(B, n, m, 0, h, mode, nullptr, &ws);
+  GatePlan gp;
+  int rc = plan_gates(mode, h, n, m, 1, 0, false, &gp);
   if (rc) return rc;
+  SolveWs ws;
+  plan_workspace(B, n, m, 0, h, gp, nullptr, &ws);
   *bytes = ws.bytes;
   return IADMM_OK;
 }
@@ -222,9 +216,10 @@ static int solve_impl(const void* packed_weights, const float* Q, const float* p
     IADMM_FAIL(IADMM_EALIGN, "solve: H, C, workspace and packed weights must be 16-byte aligned");
   int rc = check_device();
   if (rc) return rc;
+  GatePlan gp;
+  if ((rc = plan_gates(mode, h, n, m, K, flags, false, &gp))) return rc;
   SolveWs ws;
-  rc = plan_workspace(B, n, m, num_ineq, h, mode, workspace, &ws);
-  if (rc) return rc;
+  plan_workspace(B, n, m, num_ineq, h, gp, workspace, &ws);
   if (ws.bytes > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "solve: workspace too small: %zu < %zu", workspace_bytes, ws.bytes);
   if (K == 0) return IADMM_OK;
 
@@ -234,31 +229,21 @@ static int solve_impl(const void* packed_weights, const float* Q, const float* p
   const Sched* sched = reinterpret_cast<const Sched*>(wbase + L.off_sched);
   const float* b_h = reinterpret_cast<const float*>(wbase + L.off_bh);
   const long rows = (long)B * (n + m);
-  const bool tc = is_tc(mode);
-  const int nprod = (mode == IADMM_GATES_TC_3XFP16) ? 3 : (is_f16f8(mode) ? 2 : 1);
   const bool want_trace = pri_trace || dual_trace || pri_trace_u || dual_trace_u || metric_trace;
 
-  // small instances: one persistent CTA per instance keeps the whole iteration on chip (resident.cu)
-  if (tc && !sp && resident_eligible(n, m, h, nprod, flags))
+  if (gp.path == kGatesResident)
     return launch_solve_resident(packed_weights, L, Q, p, A0, zl, zu, sd, se, sc, x, y, z, xv, H, C, pri_trace, dual_trace,
-                                 pri_trace_u, dual_trace_u, metric_trace, B, n, m, num_ineq, t0, K, sigma, nprod, flags, st);
+                                 pri_trace_u, dual_trace_u, metric_trace, B, n, m, num_ineq, t0, K, sigma, gp.nprod, flags, st);
 
   float* hbuf[2] = {H, ws.h_alt};
   int cur = 0;
-  // Row-interleaved state for the fused F16F8 solve (K >= 2; a single step would only pay the layout conversion):
-  // the epilogue of the gate kernel then touches whole 128-byte lines instead of one 32-byte sector per row.
-  const char* il_sw = dev_env("IADMM_TC_INTERLEAVED");     // development switch: 0 = row-major state
-  const bool keep = (flags & (IADMM_F_KEEP_PLANES | IADMM_F_RESUME)) != 0;
-  const bool il = tc && nprod == 2 && (K >= 2 || h % 16 != 0 || keep) && !(il_sw && il_sw[0] == '0') && ws.c_il != nullptr;
-  if (tc && nprod == 2 && h % 16 != 0 && !il) IADMM_FAIL(IADMM_EMODE, "hidden_dim %% 16 != 0 needs the row-interleaved fp16+fp8 kernels");
+  const bool tc = gp.path == kGatesTc, il = gp.interleaved;
   // one iteration per call (main.py:874-887): the state stays in the planes the previous call left in this workspace
   const bool resume = (flags & IADMM_F_RESUME) != 0;
-  if (resume && !il) IADMM_FAIL(IADMM_EMODE, "solve: IADMM_F_RESUME needs the row-interleaved fp16+fp8 path (iadmm_solve_state_resumable)");
   if (resume && (flags & IADMM_F_ZERO_STATE)) IADMM_FAIL(IADMM_EMODE, "solve: IADMM_F_RESUME and IADMM_F_ZERO_STATE exclude each other");
   if (resume && (flags & IADMM_F_RESUME_ODD)) cur = 1;
   TcIl ilp;
   ilp.rows_p = ws.rows_p; ilp.C_il = ws.c_il; ilp.C_rm_out = nullptr;
-  ilp.drop_h_correction = (mode == IADMM_GATES_TC_F16F8U) ? 1 : 0;
   if (il) {
     const size_t hb = (size_t)ws.rows_p * h * sizeof(__half);
     const size_t qb = il_q8_bytes(ws.rows_p, h);
@@ -277,11 +262,11 @@ static int solve_impl(const void* packed_weights, const float* Q, const float* p
       if ((rc = launch_c_to_il(C, ws.c_il, rows, h, st))) return rc;
     }
   } else if (tc) {
-    if (flags & IADMM_F_ZERO_STATE) rc = launch_zero_state(ws.tc.h_hi[0], ws.tc.h_lo[0], rows, h, nprod, st);
-    else                            rc = launch_split_state(H, ws.tc.h_hi[0], ws.tc.h_lo[0], rows, h, nprod, st);
+    if (flags & IADMM_F_ZERO_STATE) rc = launch_zero_state(ws.tc.h_hi[0], ws.tc.h_lo[0], rows, h, gp.nprod, st);
+    else                            rc = launch_split_state(H, ws.tc.h_hi[0], ws.tc.h_lo[0], rows, h, gp.nprod, st);
     if (rc) return rc;
     // the other ping-pong buffer: padding bytes of the packed e4m3 rows must be finite (never multiplied, but loaded)
-    if (nprod == 2 && K > 1) IADMM_CUDA(cudaMemsetAsync(ws.tc.h_lo[1], 0, tc_lo_bytes(rows, h), st));
+    if (gp.nprod == 2 && K > 1) IADMM_CUDA(cudaMemsetAsync(ws.tc.h_lo[1], 0, tc_lo_bytes(rows, h), st));
   }
   // programmatic dependent launches inside the KKT phase (common.cuh): measured, bit-identical and NOT faster (KKT phase 0.652 vs
   // 0.652 ms, 1.528 vs 1.522 ms at n = 5000, profiles/r02_kkt_pdl_ab.jsonl: the kernel boundaries are not where the phase loses
@@ -304,7 +289,7 @@ static int solve_impl(const void* packed_weights, const float* Q, const float* p
     if (tc) {
       ilp.C_rm_out = (k == K - 1) ? C : nullptr;
       rc = launch_gates_tc(packed_weights, L, xv, ws.s.g, ws.tc.h_hi[cur], ws.tc.h_lo[cur], ws.tc.h_hi[cur ^ 1],
-                           ws.tc.h_lo[cur ^ 1], (k == K - 1) ? H : nullptr, C, ws.head_part, rows, h, nprod, st, nullptr,
+                           ws.tc.h_lo[cur ^ 1], (k == K - 1) ? H : nullptr, C, ws.head_part, rows, h, gp, st, nullptr,
                            il ? &ilp : nullptr);
     } else {
       rc = launch_gates_simt(packed_weights, L, xv, ws.s.g, hbuf[cur], hbuf[cur ^ 1], C, ws.head_part, rows, h, st);
@@ -313,7 +298,7 @@ static int solve_impl(const void* packed_weights, const float* Q, const float* p
     prof_end(kProfGates, st);
     prof_begin(kProfTail, st);
     cur ^= 1;
-    if ((rc = launch_tail(ws.d, ws.head_part, tc ? tc_head_slots(h, il, il && ilp.drop_h_correction) : ws.tiles, b_h, sk, zl, zu, x, y, z, xv, st, metric_trace ? &ws.s : nullptr))) return rc;
+    if ((rc = launch_tail(ws.d, ws.head_part, gp.head_slots, b_h, sk, zl, zu, x, y, z, xv, st, metric_trace ? &ws.s : nullptr))) return rc;
     prof_end(kProfTail, st);
   }
   if (!tc && cur == 1)
@@ -328,7 +313,9 @@ static int solve_impl(const void* packed_weights, const float* Q, const float* p
 
 int iadmm_solve_state_resumable(int n, int m, int h, int mode, int flags, int* yes) {
   if (n <= 0 || m < 0 || h <= 0 || !yes) IADMM_FAIL(IADMM_ESHAPE, "solve_state_resumable: n=%d m=%d h=%d", n, m, h);
-  *yes = (is_f16f8(mode) && h % 8 == 0 && !resident_eligible(n, m, h, 2, flags)) ? 1 : 0;
+  // IADMM_F_KEEP_PLANES asks for the row-interleaved planes wherever a path has them; an unsupported mode or shape has none
+  GatePlan gp;
+  *yes = (plan_gates(mode, h, n, m, 1, flags | IADMM_F_KEEP_PLANES, false, &gp) == IADMM_OK && gp.interleaved) ? 1 : 0;
   return IADMM_OK;
 }
 

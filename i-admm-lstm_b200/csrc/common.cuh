@@ -48,6 +48,7 @@ void set_error(const char* fmt, ...);
 constexpr int kMaxDevices = 64;
 struct PerDeviceOnce { unsigned long long done = 0ull; };     // bit d: attribute set on device d (benign if set twice)
 int device_sm_count(int* sms);                                // SM count of the CURRENT device (cached per ordinal)
+int check_device();                                           // IADMM_EARCH unless the CURRENT device is sm_100
 
 template <typename KernelT>
 static inline int ensure_dyn_smem(KernelT kernel, int bytes, PerDeviceOnce* once) {
@@ -304,7 +305,6 @@ static inline size_t q8_pitch(int h) { return (size_t)((h + 63) / 64) * 128; }
 // fp16(U*2^s) < 2^13 -> *2^-5 < 256; residual of U*2^s is < 2 -> *2^6 < 128  (e4m3 max = 448)
 constexpr int kQ8HLoShift = 5, kQ8HHiShift = -6, kQ8UHiShift = -5, kQ8ULoShift = 6;
 int  tc_gate_tiles(int h);                    // head-partial slots to allocate
-int  tc_head_slots(int h, bool interleaved, bool eight_warps = false);  // slots the gate kernel writes (= what the tail sums)
 size_t tc_state_bytes(long rows, int h);
 // Row-interleaved state layout of the fused solve (F16F8 mode): every per-row array is stored [column group][row][16 or 32 B]
 // so that the thread-per-row epilogue reads and writes whole 128-byte lines (see gates_tc.cu).  rows_p = rows rounded up to 128.
@@ -312,16 +312,32 @@ struct TcIl {
   long   rows_p;
   float* C_il;        // fp32 [h/8][rows_p][8], the cell state between iterations
   float* C_rm_out;    // non-NULL on the last iteration: also write the caller's row-major C [rows][h]
-  int    drop_h_correction;   // IADMM_GATES_TC_F16F8U: the e4m3 product that corrects the fp16 rounding of H is not issued
 };
 static inline long il_rows(long rows) { return (rows + 127) / 128 * 128; }
 // bytes of one row-interleaved e4m3 plane pair [ceil(h/16)][residual | coarse][rows_p][16]; with hidden_dim % 16 == 8 the last
 // 16-unit group is half padding, which must read as zero (it is multiplied)
 static inline size_t il_q8_bytes(long rows_p, int h) { return (size_t)((h + 15) / 16) * 2 * (size_t)rows_p * 16; }
+
+// The gate-contraction path of one call: which kernels run, with how many products, and how many head partials per row the
+// tail has to sum.  plan_gates (gates_tc.cu) is the one place that decides it; no caller compares against IADMM_GATES_*.
+enum { kGatesFp32 = 0, kGatesResident = 1, kGatesTc = 2 };
+struct GatePlan {
+  int  path;          // kGatesFp32: CUDA cores; kGatesResident: on-chip-resident solve (resident.cu); kGatesTc: streaming tensor cores
+  int  nprod;         // tensor-core products: 1 (fp16), 2 (fp16 + e4m3 corrections) or 3 (fp16 hi/lo split); 0 on CUDA cores
+  bool interleaved;   // the solve keeps its state row-interleaved between iterations (TcIl)
+  bool drop_h;        // IADMM_GATES_TC_F16F8U on the row-interleaved kernels: the e4m3 product that corrects the fp16 rounding
+                      // of H is not issued
+  int  epi_warps;     // epilogue warps of the tensor-core gate kernel (8 or 16)
+  int  head_slots;    // head partials per row the gate kernel writes = what the tail sums (0 on the resident path)
+};
+// `training`: the forward of iadmm_step_fwd / iadmm_train_window, which never runs resident or row-interleaved (K and flags
+// are then ignored).  Returns IADMM_EMODE, message set, for every mode / shape / flag combination no path serves.
+int  plan_gates(int mode, int h, int n, int m, int K, int flags, bool training, GatePlan* plan);
+
 int  launch_gates_tc(const void* packed, const WeightLayout& L, const float* xv, const float* g,
                      const __half* Hin_hi, const __half* Hin_lo, __half* Hout_hi, __half* Hout_lo,
                      float* H_out_f32 /* may be NULL */, float* C, float* head_part, long rows, int h,
-                     int nprod, cudaStream_t st, float* gates_out = nullptr, const TcIl* il = nullptr);
+                     const GatePlan& plan, cudaStream_t st, float* gates_out = nullptr, const TcIl* il = nullptr);
 int  launch_split_state_il(const float* H, __half* hi, __half* q8, long rows, int h, cudaStream_t st);
 int  launch_c_to_il(const float* C, float* C_il, long rows, int h, cudaStream_t st);
 int  launch_split_state(const float* H, __half* hi, __half* lo, long rows, int h, int nprod, cudaStream_t st);
@@ -329,8 +345,8 @@ int  launch_zero_state(__half* hi, __half* lo, long rows, int h, int nprod, cuda
 size_t tc_lo_bytes(long rows, int h);   // size of one `lo` buffer (fits both the fp16 and the packed e4m3 form)
 
 // O(N) tail: xv -= head ; x,z,y updates (models/lstm.py:82-94)
-// on-chip-resident solve for small instances (resident.cu)
-bool resident_eligible(int n, int m, int h, int nprod, int flags);
+// on-chip-resident solve for small instances (resident.cu): whether the shape fits it
+bool resident_eligible(int n, int m, int h, int nprod);
 int launch_solve_resident(const void* packed, const WeightLayout& L, const float* Q, const float* p, const float* A0,
                           const float* zl, const float* zu, const float* sd, const float* se, const float* sc, float* x, float* y,
                           float* z, float* xv, float* H, float* C, float* pri, float* dual, float* pri_u, float* dual_u,

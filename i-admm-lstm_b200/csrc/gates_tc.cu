@@ -1073,10 +1073,52 @@ static int select_epi_warps(int h) {
   const int env = w ? atoi(w) : 0;
   return (env == 8 || env == 16) ? env : (h <= kEpi16MaxHidden ? 16 : 8);
 }
-// head partials per launch that the tail has to sum: per unit tile one per epilogue warp slice
-int tc_head_slots(int h, bool interleaved, bool eight_warps) {
-  const bool dev_exp = dev_env("IADMM_TC_EXP") != nullptr && atoi(dev_env("IADMM_TC_EXP")) != 0;
-  return ((interleaved && !eight_warps && !dev_exp && select_epi_warps(h) == 16) ? 4 : 2) * cdiv(h, kTcUnits);
+
+int plan_gates(int mode, int h, int n, int m, int K, int flags, bool training, GatePlan* p) {
+  const bool f16f8 = mode == IADMM_GATES_TC_F16F8 || mode == IADMM_GATES_TC_F16F8U;
+  const bool tc = f16f8 || mode == IADMM_GATES_TC_3XFP16 || mode == IADMM_GATES_TC_1XFP16;
+  if (!tc && mode != IADMM_GATES_SIMT_FP32) {
+    if (training) IADMM_FAIL(IADMM_EMODE, "training: unknown gate mode %d", mode);
+    IADMM_FAIL(IADMM_EMODE, "unknown gate mode %d", mode);
+  }
+  *p = GatePlan{kGatesFp32, 0, false, false, 0, simt_gate_tiles(h)};
+  // training runs a tensor-core mode at hidden_dim % 8 != 0 on CUDA cores; the solve rejects it
+  if (!tc || (training && h % 8 != 0)) return IADMM_OK;
+  if (h % 8 != 0) IADMM_FAIL(IADMM_EMODE, "tensor-core gate modes need hidden_dim %% 8 == 0 (got %d)", h);
+  p->path = kGatesTc;
+  p->nprod = (mode == IADMM_GATES_TC_3XFP16) ? 3 : (mode == IADMM_GATES_TC_1XFP16) ? 1 : 2;
+  p->epi_warps = kTcEpiWarps;
+  if (training) {
+    // both corrections of the F16F8 modes are kept; at hidden_dim % 16 == 8 as the 3-way split, since only the row-interleaved
+    // kernels pad the last 16-unit e4m3 group
+    if (f16f8 && h % 16 != 0) p->nprod = 3;
+  } else {
+    // small instances: one persistent CTA per instance keeps the whole iteration on chip (F16F8U runs full F16F8 there)
+    const char* res_sw = dev_env("IADMM_RESIDENT");            // development switch: 0 = always the streaming path
+    if (!(flags & IADMM_F_STREAMING) && !(res_sw && res_sw[0] == '0') && resident_eligible(n, m, h, p->nprod)) {
+      p->path = kGatesResident;
+      p->epi_warps = p->head_slots = 0;
+      return IADMM_OK;
+    }
+    // Row-interleaved state for the fused F16F8 solve (K >= 2; a single step would only pay the layout conversion, unless the
+    // caller keeps the planes for the next call): the epilogue of the gate kernel then touches whole 128-byte lines instead of
+    // one 32-byte sector per row.  With hidden_dim % 16 == 8 only these kernels pad the last 16-unit e4m3 group.
+    const char* il_sw = dev_env("IADMM_TC_INTERLEAVED");       // development switch: 0 = row-major state
+    const bool keep = (flags & (IADMM_F_KEEP_PLANES | IADMM_F_RESUME)) != 0;
+    p->interleaved = f16f8 && (K >= 2 || h % 16 != 0 || keep) && !(il_sw && il_sw[0] == '0');
+    if (f16f8 && h % 16 != 0 && !p->interleaved) IADMM_FAIL(IADMM_EMODE, "hidden_dim %% 16 != 0 needs the row-interleaved fp16+fp8 kernels");
+    if ((flags & IADMM_F_RESUME) && !p->interleaved)
+      IADMM_FAIL(IADMM_EMODE, "solve: IADMM_F_RESUME needs the row-interleaved fp16+fp8 path (iadmm_solve_state_resumable)");
+    p->drop_h = p->interleaved && mode == IADMM_GATES_TC_F16F8U;
+    // the F16F8U product set and the IADMM_TC_EXP ablations exist only in the 8-warp instantiation
+    const char* exp_sw = dev_env("IADMM_TC_EXP");
+    if (p->interleaved && !p->drop_h && !(exp_sw && atoi(exp_sw) != 0)) p->epi_warps = select_epi_warps(h);
+  }
+  // one head partial per unit tile and epilogue warp slice of four warps
+  p->head_slots = p->epi_warps / 4 * cdiv(h, kTcUnits);
+  if (p->head_slots > tc_gate_tiles(h))
+    IADMM_FAIL(IADMM_EMODE, "gate plan: %d head partials per row exceed the %d workspace slots", p->head_slots, tc_gate_tiles(h));
+  return IADMM_OK;
 }
 
 static bool use_quads() {
@@ -1093,7 +1135,9 @@ static bool use_cta_pairs() {
 
 int launch_gates_tc(const void* packed, const WeightLayout& L, const float* xv, const float* g, const __half* Hin_hi,
                     const __half* Hin_lo, __half* Hout_hi, __half* Hout_lo, float* H_out_f32, float* C,
-                    float* head_part, long rows, int h, int nprod, cudaStream_t st, float* gates_out, const TcIl* il) {
+                    float* head_part, long rows, int h, const GatePlan& plan, cudaStream_t st, float* gates_out, const TcIl* il) {
+  const int nprod = plan.nprod;
+  if (plan.interleaved != (il != nullptr)) IADMM_FAIL(IADMM_EMODE, "gate plan and row-interleaved state buffers disagree");
   if (h % 8 != 0) IADMM_FAIL(IADMM_EMODE, "tensor-core gate path needs hidden_dim %% 8 == 0");
   if (rows > 0x7fffffffL - 2 * kTcBM) IADMM_FAIL(IADMM_ESHAPE, "too many rows for one launch");
   int num_sms = 0, rc;
@@ -1154,9 +1198,8 @@ int launch_gates_tc(const void* packed, const WeightLayout& L, const float* xv, 
     if (epi < 0 || epi > 3) epi = 1;                  // 3: shared-reciprocal activations (row-interleaved kernel only)
   }
   // IADMM_GATES_TC_F16F8U: the H-rounding correction product is not issued (TcParams::exp 7 is exactly that and numerically valid)
-  const bool drop_h = il && il->drop_h_correction;
-  if (drop_h && exp_mode == 0) exp_mode = 7;
-  const int epi_warps = (drop_h || exp_mode) ? 8 : select_epi_warps(h);     // the switch lives in the 8-warp instantiation
+  if (plan.drop_h && exp_mode == 0) exp_mode = 7;
+  const int epi_warps = plan.epi_warps;
   P.exp = exp_mode;
   if (const char* e = dev_env("IADMM_TC_WAIT_NS")) P.wait_ns = (uint32_t)atoi(e);
   // cluster size: 4 (two pairs sharing each U tile through TMA multicast) when there is enough work, else 2

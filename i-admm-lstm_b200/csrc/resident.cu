@@ -581,9 +581,7 @@ __global__ void __launch_bounds__(kResThreads, 1) solve_resident_kernel(const Re
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-bool resident_eligible(int n, int m, int h, int nprod, int flags) {
-  const char* e = dev_env("IADMM_RESIDENT");           // development switch: 0 = always the streaming path
-  if ((e && e[0] == '0') || (flags & IADMM_F_STREAMING)) return false;
+bool resident_eligible(int n, int m, int h, int nprod) {
   if (h != kResH || n + m > kResMaxN || nprod < 1 || nprod > 3) return false;
   return res_fixed_bytes(n, m) <= (size_t)kResSmemLimit;
 }

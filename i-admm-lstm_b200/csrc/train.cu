@@ -434,16 +434,18 @@ struct TrainWs {
   long rows_p;                                    // row count padded to 8 (pitch of the transposed operands)
   Sched* zero_sched;
   double* acc;
-  int tiles, cs_parts, cs_rows;
+  int cs_parts, cs_rows;
   size_t bytes;
 };
 
 static void plan_train(int B, int n, int m, int num_ineq, int h, void* base, TrainWs* W) {
   W->d = make_kkt_dims_train(B, n, m, num_ineq);
   const size_t rows = (size_t)B * (n + m);
-  W->tiles = simt_gate_tiles(h);
-  const int tc_tiles = (h % 8 == 0) ? tc_gate_tiles(h) : 0;
-  const int max_tiles = W->tiles > tc_tiles ? W->tiles : tc_tiles;
+  // sized for every gate mode: the tensor-core images and head slots exist where a tensor-core mode runs at this hidden_dim
+  GatePlan tc;
+  const bool tc_fwd = plan_gates(IADMM_GATES_TC_3XFP16, h, n, m, 1, 0, true, &tc) == IADMM_OK && tc.path == kGatesTc;
+  const int simt_tiles = simt_gate_tiles(h), tc_tiles = tc_fwd ? tc_gate_tiles(h) : 0;
+  const int max_tiles = simt_tiles > tc_tiles ? simt_tiles : tc_tiles;
   W->cs_rows = cs_rows_per_part(rows);
   W->cs_parts = (int)((rows + W->cs_rows - 1) / W->cs_rows);
   char* p = static_cast<char*>(base);
@@ -453,7 +455,7 @@ static void plan_train(int B, int n, int m, int num_ineq, int h, void* base, Tra
   if (base) kkt_scratch_carve(W->d, kkt, &W->s);
   W->head_part = reinterpret_cast<float*>(take((size_t)max_tiles * rows * sizeof(float)));
   W->h_hi = W->h_lo = W->h_hi_out = W->h_lo_out = nullptr;
-  if (h % 8 == 0) {
+  if (tc_fwd) {
     W->h_hi = reinterpret_cast<__half*>(take(rows * (size_t)h * sizeof(__half)));
     W->h_lo = reinterpret_cast<__half*>(take(tc_lo_bytes((long)rows, h)));
     W->h_hi_out = reinterpret_cast<__half*>(take(rows * (size_t)h * sizeof(__half)));
@@ -488,39 +490,21 @@ static void plan_train(int B, int n, int m, int num_ineq, int h, void* base, Tra
   W->bytes = off;
 }
 
-static int check_sm100() {
-  int dev = 0, major = 0;
-  IADMM_CUDA(cudaGetDevice(&dev));
-  IADMM_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-  if (major != 10) IADMM_FAIL(IADMM_EARCH, "device %d has compute capability %d.x; libiadmm_b200 needs sm_100 (B200)", dev, major);
-  return IADMM_OK;
-}
-
-
 // The forward gate contraction + cell of one training iteration (fp32 CUDA cores, or the tensor-core kernel with the state
 // converted at the boundary), keeping the gate activations.  C_o must already hold C (the cell kernels update it in place).
-// Returns the number of head partials written per row through *head_slots.
+// Writes gp.head_slots head partials per row.
 static int train_gate_forward(const void* packed_weights, const WeightLayout& L, const TrainWs& W, const float* xv, const float* g,
-                              const float* H, float* H_o, float* C_o, float* gates_out, size_t rows, int h, int mode,
-                              int* head_slots, cudaStream_t st) {
+                              const float* H, float* H_o, float* C_o, float* gates_out, size_t rows, int h, const GatePlan& gp,
+                              cudaStream_t st) {
   int rc;
-  int nprod = 0;
-  if (mode == IADMM_GATES_TC_3XFP16 && h % 8 == 0) nprod = 3;
-  else if ((mode == IADMM_GATES_TC_F16F8 || mode == IADMM_GATES_TC_F16F8U) && h % 16 == 0) nprod = 2;   // training keeps both corrections
-  else if ((mode == IADMM_GATES_TC_F16F8 || mode == IADMM_GATES_TC_F16F8U) && h % 8 == 0) nprod = 3;
-  else if (mode == IADMM_GATES_TC_1XFP16 && h % 8 == 0) nprod = 1;
-  else if (mode != IADMM_GATES_SIMT_FP32 && h % 8 == 0) IADMM_FAIL(IADMM_EMODE, "training: unknown gate mode %d", mode);
-  if (nprod == 0) {
-    *head_slots = W.tiles;
+  if (gp.path == kGatesFp32)
     return launch_gates_simt(packed_weights, L, xv, g, H, H_o, C_o, W.head_part, (long)rows, h, st, gates_out);
-  }
   prof_begin(kProfTrainGates, st);
-  if ((rc = launch_split_state(H, W.h_hi, W.h_lo, (long)rows, h, nprod, st))) return rc;
-  if (nprod == 2) IADMM_CUDA(cudaMemsetAsync(W.h_lo_out, 0, tc_lo_bytes((long)rows, h), st));
+  if ((rc = launch_split_state(H, W.h_hi, W.h_lo, (long)rows, h, gp.nprod, st))) return rc;
+  if (gp.nprod == 2) IADMM_CUDA(cudaMemsetAsync(W.h_lo_out, 0, tc_lo_bytes((long)rows, h), st));
   if ((rc = launch_gates_tc(packed_weights, L, xv, g, W.h_hi, W.h_lo, W.h_hi_out, W.h_lo_out, H_o, C_o, W.head_part,
-                            (long)rows, h, nprod, st, gates_out))) return rc;
+                            (long)rows, h, gp, st, gates_out))) return rc;
   prof_end(kProfTrainGates, st);
-  *head_slots = tc_head_slots(h, false);
   return IADMM_OK;
 }
 
@@ -556,8 +540,10 @@ int iadmm_step_fwd(const void* packed_weights, const float* Q, const float* p, c
   if (!packed_weights || !Q || !p || !x || !xv || !H || !C || !x_o || !xv_o || !H_o || !C_o || !g_save || !w_save || !workspace)
     IADMM_FAIL(IADMM_EALIGN, "step_fwd: NULL pointer");            // gates_save may be NULL: activations not kept
   if (h % 4 != 0) IADMM_FAIL(IADMM_ESHAPE, "step_fwd: hidden_dim %% 4 != 0 not supported by the training path");
-  int rc = check_sm100();
+  int rc = check_device();
   if (rc) return rc;
+  GatePlan gp;
+  if ((rc = plan_gates(mode, h, n, m, 1, 0, true, &gp))) return rc;
   TrainWs W;
   plan_train(B, n, m, num_ineq, h, workspace, &W);
   if (W.bytes > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "step_fwd: workspace too small: %zu < %zu", workspace_bytes, W.bytes);
@@ -586,9 +572,8 @@ int iadmm_step_fwd(const void* packed_weights, const float* Q, const float* p, c
   prof_end(kProfTrainKkt, st);
   // gate contraction of the forward: fp32 CUDA cores, or the tensor-core kernel (same arithmetic as the solve) with
   // the state converted at the boundary; both keep the gate activations for the backward
-  int head_slots = 0;
-  if ((rc = train_gate_forward(packed_weights, L, W, xv, W.s.g, H, H_o, C_o, gates_save, rows, h, mode, &head_slots, st))) return rc;
-  return launch_tail(W.d, W.head_part, head_slots, b_h, sk, zl, zu, x_o, y_o, z_o, xv_o, st);
+  if ((rc = train_gate_forward(packed_weights, L, W, xv, W.s.g, H, H_o, C_o, gates_save, rows, h, gp, st))) return rc;
+  return launch_tail(W.d, W.head_part, gp.head_slots, b_h, sk, zl, zu, x_o, y_o, z_o, xv_o, st);
 }
 
 int iadmm_step_bwd(const void* packed_weights, const float* Q, const float* p, const float* A0, const float* zl,
@@ -607,7 +592,7 @@ int iadmm_step_bwd(const void* packed_weights, const float* Q, const float* p, c
     IADMM_FAIL(IADMM_EALIGN, "step_bwd: NULL pointer");
   if (m > 0 && (!gy || !gz || !y || !z || !A0 || !zl || !zu)) IADMM_FAIL(IADMM_EALIGN, "step_bwd: NULL constraint pointer");
   if (h % 4 != 0) IADMM_FAIL(IADMM_ESHAPE, "step_bwd: hidden_dim %% 4 != 0 not supported by the training path");
-  int rc = check_sm100();
+  int rc = check_device();
   if (rc) return rc;
   TrainWs W;
   plan_train(B, n, m, num_ineq, h, workspace, &W);
@@ -785,7 +770,7 @@ int iadmm_residuals_fwd(const float* x, const float* y, const float* z, const fl
   if (B <= 0 || n <= 0 || m < 0 || B > 65535) IADMM_FAIL(IADMM_ESHAPE, "residuals_fwd: B=%d n=%d m=%d", B, n, m);
   if (!x || !Q || !p || !pri || !dual || !rd_save || !workspace) IADMM_FAIL(IADMM_EALIGN, "residuals_fwd: NULL pointer");
   if (m > 0 && (!y || !z || !A0 || !rp_save)) IADMM_FAIL(IADMM_EALIGN, "residuals_fwd: NULL constraint pointer");
-  int rc = check_sm100();
+  int rc = check_device();
   if (rc) return rc;
   const KktDims d = make_kkt_dims_train(B, n, m, 0);
   if (kkt_scratch_floats(d) * sizeof(float) > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "residuals_fwd: workspace too small");
@@ -809,7 +794,7 @@ int iadmm_residuals_bwd(const float* Q, const float* A0, const float* pri, const
   if (B <= 0 || n <= 0 || m < 0 || B > 65535) IADMM_FAIL(IADMM_ESHAPE, "residuals_bwd: B=%d n=%d m=%d", B, n, m);
   if (!Q || !pri || !dual || !rd_save || !gx || !workspace) IADMM_FAIL(IADMM_EALIGN, "residuals_bwd: NULL pointer");
   if (m > 0 && (!A0 || !rp_save || !gy || !gz)) IADMM_FAIL(IADMM_EALIGN, "residuals_bwd: NULL constraint pointer");
-  int rc = check_sm100();
+  int rc = check_device();
   if (rc) return rc;
   const KktDims d = make_kkt_dims_train(B, n, m, 0);
   const size_t need = kkt_scratch_floats(d) * sizeof(float) + 1024;
@@ -951,6 +936,9 @@ int iadmm_train_window(const void* packed_weights, const float* Q, const float* 
   if (!packed_weights || !Q || !p || !x || !xv || !H || !C || !grad_flat || !loss_out || !workspace)
     IADMM_FAIL(IADMM_EALIGN, "train_window: NULL pointer");
   if (m > 0 && (!A0 || !zl || !zu || !y || !z)) IADMM_FAIL(IADMM_EALIGN, "train_window: NULL constraint pointer");
+  GatePlan gp;
+  int rc = plan_gates(mode, h, n, m, 1, 0, true, &gp);
+  if (rc) return rc;
   const bool recompute = (flags & IADMM_TRAIN_RECOMPUTE_GATES) != 0;
   WindowWs W;
   plan_window(B, n, m, h, TL, flags, workspace, &W);
@@ -958,7 +946,6 @@ int iadmm_train_window(const void* packed_weights, const float* Q, const float* 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const size_t N = (size_t)n + m, rows = (size_t)B * N, fb = sizeof(float);
   const size_t sx = (size_t)B * n, sy = (size_t)B * m, sxv = rows, sH = rows * h, sG = rows * 4 * h;
-  int rc;
   // state 0 = the caller's state
   IADMM_CUDA(cudaMemcpyAsync(W.x, x, sx * fb, cudaMemcpyDeviceToDevice, st));
   if (m > 0) {
@@ -1011,9 +998,8 @@ int iadmm_train_window(const void* packed_weights, const float* Q, const float* 
       plan_train(B, n, m, num_ineq, h, W.step_ws, &T);
       const WeightLayout Lw = weight_layout(h, length);
       IADMM_CUDA(cudaMemcpyAsync(W.Cs, W.C + a * sH, sH * fb, cudaMemcpyDeviceToDevice, st));
-      int slots = 0;
       if ((rc = train_gate_forward(packed_weights, Lw, T, W.xv + a * sxv, W.g_save + a * sxv, W.H + a * sH, W.Hs, W.Cs, W.gates,
-                                   rows, h, mode, &slots, st))) return rc;
+                                   rows, h, gp, st))) return rc;
       gates_t = W.gates;
     }
     if ((rc = iadmm_step_bwd(packed_weights, Q, p, A0, zl, zu, W.x + a * sx, W.y + a * sy, W.z + a * sy, W.xv + a * sxv, W.H + a * sH,

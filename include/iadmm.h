@@ -51,18 +51,22 @@ enum {
 enum {
   IADMM_GATES_SIMT_FP32   = 0,  /* fp32 FMA on CUDA cores: bit-stable validation path                   */
   IADMM_GATES_TC_3XFP16   = 1,  /* tcgen05, fp16 hi/lo split of both operands, 3 MMAs, fp32 accumulate: */
-                                /* ~22-bit operands, the default (parity <= 1e-4 after K=100)           */
+                                /* ~22-bit operands (parity <= 1e-4 after K=100)                        */
   IADMM_GATES_TC_1XFP16   = 2,  /* tcgen05, single fp16 MMA (TF32-class operands): opt-in fast mode     */
   IADMM_GATES_TC_F16F8    = 3,  /* tcgen05, fp16 main product + two fp8 (e4m3) correction products for  */
                                 /* the operand rounding residuals: ~16-bit operands at 2/3 of the cost  */
                                 /* of the 3-way split: THE DEFAULT.  hidden_dim % 8 == 0; with           */
                                 /* hidden_dim % 16 == 8 (configs/QP.yaml's 200) the solve pads the last */
                                 /* 16-unit operand group, training uses the 3-way split                  */
-  IADMM_GATES_TC_F16F8U   = 4   /* opt-in: as F16F8 but only the rounding of the WEIGHTS U is corrected */
-                                /* (1.5 instead of 2 MMA units in the fused K >= 2 solve; single steps  */
-                                /* and training run F16F8).  The fp16 rounding of H then acts as fresh  */
-                                /* 2^-12 noise every iteration: K=100 parity measured at 1e-5..5e-5,    */
-                                /* inside the 1e-4 bar with a 2x (not 20x) margin -- see DESIGN.md      */
+  IADMM_GATES_TC_F16F8U   = 4   /* opt-in: as F16F8, but wherever the solve keeps its state             */
+                                /* row-interleaved only the rounding of the WEIGHTS U is corrected (1.5 */
+                                /* instead of 2 MMA units): the HBM-streaming solve with K >= 2, with   */
+                                /* hidden_dim % 16 == 8, or with IADMM_F_KEEP_PLANES / IADMM_F_RESUME   */
+                                /* (LSTM.forward's steps on that path).  The on-chip-resident solve,    */
+                                /* the other K = 1 calls and training run F16F8 exactly.  The fp16      */
+                                /* rounding of H then acts as fresh 2^-12 noise every iteration: K=100  */
+                                /* parity measured at 1e-5..5e-5, inside the 1e-4 bar with a 2x (not    */
+                                /* 20x) margin -- see DESIGN.md                                         */
 };
 
 /* Flags of iadmm_solve. */
@@ -141,7 +145,8 @@ int iadmm_ruiz(const float* Q, const float* p, const float* A0, const float* zl,
  */
 int iadmm_solve_workspace_bytes(int B, int n, int m, int h, int mode, size_t* bytes);
 /* *yes = 1 when iadmm_solve honours IADMM_F_KEEP_PLANES / IADMM_F_RESUME for this shape and mode (the fp16+fp8 modes on the
- * HBM-streaming path), else 0: the flags are then ignored and H, C are read on entry as usual. */
+ * HBM-streaming path), else 0: IADMM_F_KEEP_PLANES is then ignored and H, C are read on entry as usual; IADMM_F_RESUME is
+ * ignored by the on-chip-resident path and rejected with IADMM_EMODE elsewhere. */
 int iadmm_solve_state_resumable(int n, int m, int h, int mode, int flags, int* yes);
 int iadmm_solve(const void* packed_weights,
                 const float* Q, const float* p, const float* A0, const float* zl, const float* zu,
@@ -232,9 +237,10 @@ int iadmm_lu_solve(const float* LU, const int* perm, float* rhs, int B, int N, v
  * primal_dual_loss (utils.py:68-71) in the training loop main.py:336-358.  One differentiable iteration =
  * iadmm_step_fwd (out of place, saves g = K^T(K xv - rhs), w = K xv - rhs and the gate activations) +
  * iadmm_step_bwd (hand-written adjoint; reuses the two streaming KKT passes, two fp32 GEMMs for the gate
- * products).  The forward gate contraction runs in `mode` (IADMM_GATES_*, tensor cores by default like the solve);
- * the backward is fp32 CUDA-core arithmetic.  Adam (main.py:191) stays in PyTorch; data-parallel
- * training all-reduces the flat gradient buffer over NCCL (iadmm_b200/dist.py).
+ * products).  The forward gate contraction runs in `mode` (IADMM_GATES_*, tensor cores by default like the solve;
+ * F16F8 and F16F8U both keep the two correction products, as the 3-way split at hidden_dim % 16 == 8; a tensor-core mode
+ * runs fp32 at hidden_dim % 8 != 0; an unknown mode is IADMM_EMODE); the backward is fp32 CUDA-core arithmetic.  Adam
+ * (main.py:191) stays in PyTorch; data-parallel training all-reduces the flat gradient buffer over NCCL (iadmm_b200/dist.py).
  *
  * grad_flat: [iadmm_param_count] floats in state_dict order (W_i,U_i,b_i, W_f,.., W_u,U_u,b_u, W_h, b_h, rho,
  * alpha); iadmm_step_bwd ADDS this iteration's parameter adjoints to it.  Incoming adjoints g*_o may be

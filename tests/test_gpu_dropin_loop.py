@@ -51,11 +51,13 @@ def call(model, t, mi, me, st, data):
 
 
 # hidden_dim 400: the 8-warp production kernel <2,2,4> (hidden_dim > 384); 320: the 16-warp kernel <2,2,9>; 200: its padded last
-# operand group (hidden_dim % 16 == 8); 64 with n + m > 256: the 16-warp kernel on the streaming path
+# operand group (hidden_dim % 16 == 8); 64 with n + m > 256: the 16-warp kernel on the streaming path.  tc_f16f8u drops the
+# H-rounding correction on the row-interleaved path, which both the single steps and the fused solve take (8-warp kernel <2,2,4>)
+@pytest.mark.parametrize("mode", ["tc_f16f8", "tc_f16f8u"])
 @pytest.mark.parametrize("h,n,mi,me", [(400, 70, 13, 29), (320, 48, 16, 16), (200, 64, 32, 32), (64, 200, 60, 60)])
-def test_forward_loop_equals_fused_solve(h, n, mi, me):
+def test_forward_loop_equals_fused_solve(h, n, mi, me, mode):
     B, K, m = 3, 6, mi + me
-    model, prm = make(h, K)
+    model, prm = make(h, K, mode)
     data = scaled_qp(B, n, mi, me, seed=31)
     with torch.no_grad():
         fused = model.solve(K, mi, me, *data, SIGMA, traces=False)

@@ -141,7 +141,7 @@ def test_residual_gradients():
     assert rel_err(xg.grad, xr.grad) < 1e-5 and rel_err(yg.grad, yr.grad) < 1e-5 and rel_err(zg.grad, zr.grad) < 1e-5
 
 
-@pytest.mark.parametrize("mode", ["simt_fp32", "tc_f16f8"])
+@pytest.mark.parametrize("mode", ["simt_fp32", "tc_f16f8", "tc_f16f8u"])
 @pytest.mark.parametrize("shape", [(3, 24, 7, 9, 16, 6), (2, 37, 9, 11, 48, 5), (2, 20, 0, 0, 16, 4)])
 def test_fused_window_equals_per_iteration_autograd(shape, mode):
     """iadmm_train_window (one call per window) against the per-iteration autograd path it replaces: same kernels in
