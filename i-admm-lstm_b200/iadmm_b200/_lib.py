@@ -52,6 +52,8 @@ SIGNATURES = {
     "iadmm_kkt_penalty_diagonal": ([_P, _P] + [_I] * 7 + [_P], c_int),
     "iadmm_lu_factor": ([_P] * 4 + [_I, _I, _P], c_int),
     "iadmm_lu_solve": ([_P] * 3 + [_I, _I, _P], c_int),
+    "iadmm_lu_factor_blocked_workspace_bytes": ([_I, _I, POINTER(_Z)], c_int),
+    "iadmm_lu_factor_blocked": ([_P] * 4 + [_I, _I, _P, _Z, _P], c_int),
     "iadmm_param_count": ([_I, _I, POINTER(_Z)], c_int),
     "iadmm_train_workspace_bytes": ([_I, _I, _I, _I, POINTER(_Z)], c_int),
     "iadmm_step_fwd": ([_P] * 21 + [_I] * 7 + [_F, _I, _P, _Z, _P], c_int),

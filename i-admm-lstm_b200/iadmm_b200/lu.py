@@ -3,20 +3,26 @@
 Stage II is OUTSIDE the accelerated path (SURVEY.md section 8 row f1): it is exact OSQP-style ADMM, one dense LU of
 the KKT matrix and a triangular solve per iteration.  This module keeps `main.py --feas_rest` working on a B200
 next to the drop-in `LSTM`/`Scaling`.  The factorisation (`iadmm_lu_factor`, csrc/lu.cu: register-resident
-16-column panels, partial pivoting with LAPACK's first-maximum rule) and the per-iteration triangular solves
-(`iadmm_lu_solve`) are the library's own kernels; the K matrix comes from `LSTM.forward`'s return tuple
+16-column panels, partial pivoting with LAPACK's first-maximum rule, N <= 4096; above that `iadmm_lu_factor_blocked`:
+128-column blocks, cluster-wide pivot search and a 3xTF32 tensor-core trailing update, N <= 32768) and the
+per-iteration triangular solves (`iadmm_lu_solve`) are the library's own kernels; the K matrix comes from `LSTM.forward`'s return tuple
 (`iadmm_build_kkt`).  `lu`/`piv` in the return tuple are opaque to the caller exactly as in the reference
 (main.py only hands them back): `lu` is the packed L\\U factor [B,N,N], `piv` an int32 tensor [2,B,N] holding
 the interchange sequence and the row permutation derived from it.
 """
+from ctypes import byref, c_size_t
+
 import torch
 import torch.nn as nn
 
 from . import _lib
 
+REGISTER_PANEL_MAX_N = 4096          # iadmm_lu_factor's limit: one CTA holds a 16-column panel in registers
+
 
 def lu_factor(K):
-    """Batched LU of K [B,N,N] (fp32, CUDA).  Returns (lu, piv, info): see include/iadmm.h."""
+    """Batched LU of K [B,N,N] (fp32, CUDA), N <= 4096.  Returns (lu, piv, info): see include/iadmm.h.
+    Larger systems (up to N = 32768): `lu_factor_blocked`, same outputs."""
     _lib.require_cuda(K)
     B, N = K.shape[0], K.shape[1]
     lu = K.detach().to(torch.float32).contiguous().clone()
@@ -25,6 +31,24 @@ def lu_factor(K):
     with torch.cuda.device(K.device):
         _lib.check(_lib.lib().iadmm_lu_factor(_lib.ptr(lu), _lib.ptr(piv[0]), _lib.ptr(piv[1]), _lib.ptr(info), B, N,
                                               _lib.stream_ptr()))
+    return lu, piv, info
+
+
+def lu_factor_blocked(K):
+    """Batched LU of K [B,N,N] (fp32, CUDA) for N <= 32768: blocked, cluster-wide pivot search, 3xTF32 tensor-core
+    trailing update.  Returns (lu, piv, info) in `lu_factor`'s format (`lu_solve` takes them unchanged)."""
+    _lib.require_cuda(K)
+    B, N = K.shape[0], K.shape[1]
+    lu = K.detach().to(torch.float32).contiguous().clone()
+    piv = torch.empty(2, B, N, dtype=torch.int32, device=K.device)
+    info = torch.empty(B, dtype=torch.int32, device=K.device)
+    L = _lib.lib()
+    nbytes = c_size_t()
+    _lib.check(L.iadmm_lu_factor_blocked_workspace_bytes(B, N, byref(nbytes)))
+    ws = _lib.workspace(nbytes.value, K.device)
+    with torch.cuda.device(K.device):
+        _lib.check(L.iadmm_lu_factor_blocked(_lib.ptr(lu), _lib.ptr(piv[0]), _lib.ptr(piv[1]), _lib.ptr(info), B, N,
+                                             _lib.ptr(ws), nbytes.value, _lib.stream_ptr()))
     return lu, piv, info
 
 
@@ -59,7 +83,10 @@ class LU(nn.Module):
                 top = torch.cat((Q + sigma * torch.eye(n, device=Q.device), A0.transpose(1, 2)), dim=2)
                 bot = torch.cat((A0, torch.diag_embed(-inv_rho.squeeze(-1))), dim=2)
                 A_tild = torch.cat((top, bot), dim=1)
-            lu, piv, _ = lu_factor(A_tild)
+            if A_tild.shape[-1] <= REGISTER_PANEL_MAX_N:
+                lu, piv, _ = lu_factor(A_tild)
+            else:
+                lu, piv, _ = lu_factor_blocked(A_tild)
         xv = lu_solve(lu, piv, b_tild)
         n = x.shape[1]
         x_tild, v = xv[:, :n, :], xv[:, n:, :]

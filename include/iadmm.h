@@ -225,8 +225,22 @@ int iadmm_kkt_penalty_diagonal(const void* packed_weights, float* Kmat, int B, i
  * Replaces: `torch.lu(A_tild, pivot=True)` (models/lu.py:30) -- LAPACK getrf semantics, partial pivoting,
  * first maximum.  Kmat [B,N,N] row-major is overwritten by L (unit, below the diagonal) and U; piv [B,N] is
  * the 0-based interchange sequence, perm [B,N] the resulting row permutation (row i of P*K = row perm[i] of
- * K), info [B] (may be NULL) is 0 or 1 + the index of the first exactly-zero pivot.  N <= 4096. */
+ * K), info [B] (may be NULL) is 0 or 1 + the index of the first exactly-zero pivot.  N <= 4096 (its 16-column
+ * panel is held in the registers of one CTA); larger systems go to iadmm_lu_factor_blocked. */
 int iadmm_lu_factor(float* Kmat, int* piv, int* perm, int* info, int B, int N, void* stream);
+
+/* The same factorisation for 1 <= N <= 32768 (B <= 65535), with the same outputs and semantics, so iadmm_lu_solve
+ * consumes them unchanged.  Blocked right-looking LU with 128-column outer blocks: each 16-column sub-panel runs on a
+ * thread-block cluster of up to 8 CTAs (4096 rows each) that agree on every pivot through distributed shared memory;
+ * the trailing update A22 -= L21 U12 runs on the tensor cores as three tf32 products (hi*hi + hi*lo + lo*hi of a tf32
+ * hi/lo split of both operands, fp32 accumulation), ~fp32 accuracy without scaling.  Results are deterministic, but
+ * not bit-identical to iadmm_lu_factor's (the update order differs).  `workspace` holds the split operands; its size
+ * comes from iadmm_lu_factor_blocked_workspace_bytes and its contents on entry do not matter.
+ * Errors: IADMM_EMODE for N > 32768, IADMM_EWORK for a short workspace, IADMM_EALIGN for NULL pointers (info may be
+ * NULL), IADMM_EARCH off sm_100. */
+int iadmm_lu_factor_blocked_workspace_bytes(int B, int N, size_t* bytes);
+int iadmm_lu_factor_blocked(float* Kmat, int* piv, int* perm, int* info, int B, int N,
+                            void* workspace, size_t workspace_bytes, void* stream);
 
 /* Replaces: `torch.lu_solve(b_tild, lu, piv)` (models/lu.py:35), once per Stage-II iteration.
  * rhs [B,N] is overwritten by the solution. */
