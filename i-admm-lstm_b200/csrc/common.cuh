@@ -331,8 +331,20 @@ struct GatePlan {
   int  head_slots;    // head partials per row the gate kernel writes = what the tail sums (0 on the resident path)
 };
 // `training`: the forward of iadmm_step_fwd / iadmm_train_window, which never runs resident or row-interleaved (K and flags
-// are then ignored).  Returns IADMM_EMODE, message set, for every mode / shape / flag combination no path serves.
+// are then ignored) and is planned at the width train_hidden(h).  Returns IADMM_EMODE, message set, for every mode / shape /
+// flag combination no path serves.
 int  plan_gates(int mode, int h, int n, int m, int K, int flags, bool training, GatePlan* plan);
+// The width the training kernels run a model of hidden_dim h at: h rounded up to 4.  Units h..hp-1 get zero weights and a
+// zero state; their gates are then 0.5, 0.5, 0.5, tanh(0) = 0, so C and H stay exactly 0 and, with zero U rows and W_h
+// entries, they add nothing to the real units: the padded model computes the same values bit for bit (train.cu).
+static inline int train_hidden(int h) { return (h + 3) / 4 * 4; }
+// pack.cu: the iadmm_pack_weights image of the model of width hp whose units h..hp-1 are zero, from an image of width h
+// (layout weight_layout(h, length)) -- byte for byte what iadmm_pack_weights writes for the zero-padded parameters into a
+// zeroed buffer, with schedule rows t_first .. t_first+sched_rows-1 of `src` as its rows 0 .. sched_rows-1.  `params`:
+// padded_param_floats(hp) floats of scratch.
+size_t padded_param_floats(int hp);
+int pack_weights_padded(const void* src, int h, int length, int t_first, int sched_rows, int hp, float* params, void* dst,
+                        cudaStream_t st);
 
 int  launch_gates_tc(const void* packed, const WeightLayout& L, const float* xv, const float* g,
                      const __half* Hin_hi, const __half* Hin_lo, __half* Hout_hi, __half* Hout_lo,

@@ -1081,6 +1081,7 @@ int plan_gates(int mode, int h, int n, int m, int K, int flags, bool training, G
     if (training) IADMM_FAIL(IADMM_EMODE, "training: unknown gate mode %d", mode);
     IADMM_FAIL(IADMM_EMODE, "unknown gate mode %d", mode);
   }
+  if (training) h = train_hidden(h);
   *p = GatePlan{kGatesFp32, 0, false, false, 0, simt_gate_tiles(h)};
   // training runs a tensor-core mode at hidden_dim % 8 != 0 on CUDA cores; the solve rejects it
   if (!tc || (training && h % 8 != 0)) return IADMM_OK;

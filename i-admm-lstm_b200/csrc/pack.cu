@@ -157,14 +157,8 @@ __global__ void __launch_bounds__(256) pack_u_kernel(PackSrc S, int h, float* __
   }
 }
 
-int pack_weights_impl(const float* const W[4], const float* const U[4], const float* const b[4], const float* W_h,
-                      const float* b_h, const float* rho, const float* alpha, int h, int length, void* packed,
-                      cudaStream_t st) {
-  const WeightLayout L = weight_layout(h, length);
-  char* base = static_cast<char*>(packed);
-  PackSrc S;
-  for (int g = 0; g < 4; ++g) { S.W[g] = W[g]; S.U[g] = U[g]; S.b[g] = b[g]; }
-  S.W_h = W_h; S.b_h = b_h; S.rho = rho; S.alpha = alpha;
+// the packing kernels into an image of layout L (width h); schedule rows are computed from S.rho / S.alpha for t < length
+static int launch_pack(const PackSrc& S, int h, int length, const WeightLayout& L, char* base, cudaStream_t st) {
   float* scale = reinterpret_cast<float*>(base + L.off_scale);
   pack_small_kernel<<<cdiv(4 * h > length ? 4 * h : length, 256), 256, 0, st>>>(
       S, h, length, reinterpret_cast<float*>(base + L.off_wc), reinterpret_cast<float*>(base + L.off_bias),
@@ -188,6 +182,80 @@ int pack_weights_impl(const float* const W[4], const float* const U[4], const fl
                                         reinterpret_cast<__half*>(base + L.off_uhi_il),
                                         reinterpret_cast<uint8_t*>(base + L.off_uq8_il), scale);
   IADMM_LAUNCH_CHECK("pack_u_kernel");
+  return IADMM_OK;
+}
+
+int pack_weights_impl(const float* const W[4], const float* const U[4], const float* const b[4], const float* W_h,
+                      const float* b_h, const float* rho, const float* alpha, int h, int length, void* packed,
+                      cudaStream_t st) {
+  PackSrc S;
+  for (int g = 0; g < 4; ++g) { S.W[g] = W[g]; S.U[g] = U[g]; S.b[g] = b[g]; }
+  S.W_h = W_h; S.b_h = b_h; S.rho = rho; S.alpha = alpha;
+  return launch_pack(S, h, length, weight_layout(h, length), static_cast<char*>(packed), st);
+}
+
+// ------------------------------------------------------------------------------------------------
+// zero-padded image for training at hidden_dim % 4 != 0 (train_hidden, common.cuh)
+// ------------------------------------------------------------------------------------------------
+// The parameter tensors of models/lstm.py:21-41 at width hp, read back from the fp32 sections of an image of width h (exact
+// copies) and zero past h.  Per gate g: W_g [2][hp], U_g [hp][hp], b_g [hp]; then W_h [hp], b_h [1].
+size_t padded_param_floats(int hp) { return 4 * ((size_t)hp * hp + 3 * (size_t)hp) + hp + 1; }
+
+__global__ void __launch_bounds__(256) unpack_padded_kernel(const float* __restrict__ u32, const float* __restrict__ wc,
+                                                            const float* __restrict__ bias, const float* __restrict__ wh,
+                                                            const float* __restrict__ bh, int h, int hp, float* __restrict__ out) {
+  const size_t H4 = 4 * (size_t)h, per_gate = (size_t)hp * hp + 3 * (size_t)hp, total = 4 * per_gate + hp + 1;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    float v = 0.f;
+    if (i < 4 * per_gate) {
+      const int g = (int)(i / per_gate);
+      size_t o = i - (size_t)g * per_gate;
+      if (o < 2 * (size_t)hp) {                                   // W_g row a, unit j
+        const int a = (int)(o / hp), j = (int)(o - (size_t)a * hp);
+        if (j < h) v = wc[a * H4 + 4 * (size_t)j + g];
+      } else if ((o -= 2 * (size_t)hp) < (size_t)hp * hp) {       // U_g [k][j]
+        const int k = (int)(o / hp), j = (int)(o - (size_t)k * hp);
+        if (k < h && j < h) v = u32[(size_t)k * H4 + 4 * (size_t)j + g];
+      } else {                                                    // b_g [j]
+        const int j = (int)(o - (size_t)hp * hp);
+        if (j < h) v = bias[4 * (size_t)j + g];
+      }
+    } else if (i < 4 * per_gate + hp) {
+      const int j = (int)(i - 4 * per_gate);
+      if (j < h) v = wh[j];
+    } else {
+      v = bh[0];
+    }
+    out[i] = v;
+  }
+}
+
+int pack_weights_padded(const void* src, int h, int length, int t_first, int sched_rows, int hp, float* params, void* dst,
+                        cudaStream_t st) {
+  const WeightLayout Ls = weight_layout(h, length), Ld = weight_layout(hp, sched_rows);
+  const char* sb = static_cast<const char*>(src);
+  char* db = static_cast<char*>(dst);
+  IADMM_CUDA(cudaMemsetAsync(dst, 0, Ld.total, st));       // the alignment gaps, as in a zeroed buffer
+  const size_t total = padded_param_floats(hp);
+  unpack_padded_kernel<<<(unsigned)((total + 255) / 256 > 1184 ? 1184 : (total + 255) / 256), 256, 0, st>>>(
+      reinterpret_cast<const float*>(sb + Ls.off_u32), reinterpret_cast<const float*>(sb + Ls.off_wc),
+      reinterpret_cast<const float*>(sb + Ls.off_bias), reinterpret_cast<const float*>(sb + Ls.off_wh),
+      reinterpret_cast<const float*>(sb + Ls.off_bh), h, hp, params);
+  IADMM_LAUNCH_CHECK("unpack_padded_kernel");
+  const size_t per_gate = (size_t)hp * hp + 3 * (size_t)hp;
+  PackSrc S;
+  for (int g = 0; g < 4; ++g) {
+    S.W[g] = params + g * per_gate;
+    S.U[g] = S.W[g] + 2 * (size_t)hp;
+    S.b[g] = S.U[g] + (size_t)hp * hp;
+  }
+  S.W_h = params + 4 * per_gate;
+  S.b_h = S.W_h + hp;
+  S.rho = S.alpha = nullptr;
+  int rc = launch_pack(S, hp, 0, Ld, db, st);               // the schedule is copied, not recomputed (the image holds no rho)
+  if (rc) return rc;
+  IADMM_CUDA(cudaMemcpyAsync(db + Ld.off_sched, sb + Ls.off_sched + (size_t)t_first * kSchedStride * sizeof(float),
+                             (size_t)sched_rows * kSchedStride * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return IADMM_OK;
 }
 

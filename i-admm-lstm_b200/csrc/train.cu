@@ -405,6 +405,58 @@ __global__ void __launch_bounds__(256) scatter_grads_kernel(int h, int t, const 
   }
 }
 
+// The same scatter for adjoints computed at the padded width hp = train_hidden(h) > h: U_bar has the row pitch 4 hp, and the
+// entries of the units h..hp-1 are dropped (the small adjoints keep the index 4 j + g).  A kernel of its own, so that the one
+// every hidden_dim % 4 == 0 runs stays as it is.
+__global__ void __launch_bounds__(256) scatter_grads_padded_kernel(int h, int hp, int t, const float* __restrict__ u32bar,
+                                                                   const float* __restrict__ w0bar, const float* __restrict__ w1bar,
+                                                                   const float* __restrict__ bbar, const float* __restrict__ whbar,
+                                                                   const float* __restrict__ sbar_sum, const double* __restrict__ acc,
+                                                                   const Sched* __restrict__ sched, GradLayout G,
+                                                                   float* __restrict__ flat) {
+  const size_t total = (size_t)h * 4 * h;
+  const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx < total) {
+    const int k = (int)(idx / (4 * (size_t)h));
+    const int c = (int)(idx - (size_t)k * 4 * h);
+    const int j = c >> 2, g = c & 3;
+    flat[G.U[g] + (size_t)k * h + j] += u32bar[(size_t)k * 4 * hp + c];
+  }
+  if (idx < (size_t)4 * h) {
+    const int j = (int)idx >> 2, g = (int)idx & 3;
+    flat[G.W[g] + j] += w0bar[idx];
+    flat[G.W[g] + h + j] += w1bar[idx];
+    flat[G.b[g] + j] += bbar[idx];
+  }
+  if (idx < (size_t)h) flat[G.W_h + idx] += whbar[idx];
+  if (idx == 0) {
+    flat[G.b_h] += sbar_sum[0];
+    const float rho = sched->rho_ineq;
+    const double rho_bar = acc[0] + 1000.0 * acc[1];
+    flat[G.rho + t] += (float)(rho_bar * (double)rho * (1.0 - (double)rho));
+    const double s = 0.5 * (double)sched->alpha;
+    flat[G.alpha + t] += (float)(acc[2] * 2.0 * s * (1.0 - s));
+  }
+}
+
+// dst [rows][dp] = src [rows][sp], columns sp..dp-1 written as 0: the caller's [rows][h] state and adjoints to the padded
+// width hp and back.  The padding columns are written every time; nothing assumes the workspace holds zeros.
+__global__ void __launch_bounds__(256) repitch_kernel(const float* __restrict__ src, int sp, float* __restrict__ dst, int dp,
+                                                      size_t count) {
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (size_t)gridDim.x * blockDim.x) {
+    const size_t r = i / dp;
+    const int j = (int)(i - r * dp);
+    dst[i] = (j < sp) ? src[r * sp + j] : 0.f;
+  }
+}
+
+static int launch_repitch(const float* src, int sp, float* dst, int dp, size_t rows, cudaStream_t st) {
+  const size_t count = rows * dp, blocks = (count + 255) / 256;
+  repitch_kernel<<<(unsigned)(blocks > 148 * 16 ? 148 * 16 : blocks), 256, 0, st>>>(src, sp, dst, dp, count);
+  IADMM_LAUNCH_CHECK("repitch_kernel");
+  return IADMM_OK;
+}
+
 __global__ void negate_sum_kernel(const float* __restrict__ Xbar, long rows, float* __restrict__ out) {
   // b_h adjoint: sum_r s_bar_r = -sum_r Xbar_r   (single block, deterministic)
   __shared__ double sh[32];
@@ -424,7 +476,28 @@ __global__ void negate_sum_kernel(const float* __restrict__ Xbar, long rows, flo
 // ------------------------------------------------------------------------------------------------
 // workspace of the training entry points
 // ------------------------------------------------------------------------------------------------
+// A call at hidden_dim h with hp = train_hidden(h) != h runs the kernels on the zero-padded model of width hp.  This holds that
+// model's weights and, for a step call, its state and adjoints; it sits at the front of the workspace.
+struct PadWs {
+  char* wimg;                                          // pack_weights_padded image (NULL when hp == h)
+  WeightLayout L;                                      // its layout: weight_layout(hp, schedule rows of the call)
+  float* params;                                       // the padded parameter tensors it is packed from
+  float *H, *C, *H_o, *C_o, *gH_o, *gC_o, *gH, *gC;    // [rows][hp] (step entry points only)
+};
+
+static void plan_pad(int h, int sched_rows, size_t rows, char* base, size_t* off, PadWs* P) {
+  const int hp = train_hidden(h);
+  auto take = [&](size_t bytes) { size_t o = *off; *off = align_up(*off + bytes, 256); return base ? base + o : nullptr; };
+  P->L = weight_layout(hp, sched_rows);
+  P->wimg = take(P->L.total);
+  P->params = reinterpret_cast<float*>(take(padded_param_floats(hp) * sizeof(float)));
+  for (float** b : {&P->H, &P->C, &P->H_o, &P->C_o, &P->gH_o, &P->gC_o, &P->gH, &P->gC})
+    *b = rows ? reinterpret_cast<float*>(take(rows * hp * sizeof(float))) : nullptr;
+}
+
 struct TrainWs {
+  int hp;                                         // the width the kernels run at: train_hidden(hidden_dim)
+  PadWs pad;                                      // step entry points at hp != hidden_dim
   KktDims d;
   KktScratch s;
   float *head_part, *zeros, *Xbar, *xvbar_cell, *gbar, *D, *u32bar, *u32bar_part, *cs_part, *w0bar, *w1bar, *bbar, *whbar, *sbar_sum;
@@ -438,9 +511,15 @@ struct TrainWs {
   size_t bytes;
 };
 
-static void plan_train(int B, int n, int m, int num_ineq, int h, void* base, TrainWs* W) {
+// Sized at the width hp = train_hidden(hidden).  `step_io`: the padded weights and state of a step call when hp != hidden.
+static void plan_train(int B, int n, int m, int num_ineq, int hidden, bool step_io, void* base, TrainWs* W) {
+  const int h = W->hp = train_hidden(hidden);
   W->d = make_kkt_dims_train(B, n, m, num_ineq);
   const size_t rows = (size_t)B * (n + m);
+  char* p = static_cast<char*>(base);
+  size_t off = 0;
+  W->pad = PadWs{};
+  if (step_io && h != hidden) plan_pad(hidden, 1, rows, p, &off, &W->pad);
   // sized for every gate mode: the tensor-core images and head slots exist where a tensor-core mode runs at this hidden_dim
   GatePlan tc;
   const bool tc_fwd = plan_gates(IADMM_GATES_TC_3XFP16, h, n, m, 1, 0, true, &tc) == IADMM_OK && tc.path == kGatesTc;
@@ -448,8 +527,6 @@ static void plan_train(int B, int n, int m, int num_ineq, int h, void* base, Tra
   const int max_tiles = simt_tiles > tc_tiles ? simt_tiles : tc_tiles;
   W->cs_rows = cs_rows_per_part(rows);
   W->cs_parts = (int)((rows + W->cs_rows - 1) / W->cs_rows);
-  char* p = static_cast<char*>(base);
-  size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return base ? p + o : nullptr; };
   float* kkt = reinterpret_cast<float*>(take(kkt_scratch_floats(W->d) * sizeof(float)));
   if (base) kkt_scratch_carve(W->d, kkt, &W->s);
@@ -508,52 +585,18 @@ static int train_gate_forward(const void* packed_weights, const WeightLayout& L,
   return IADMM_OK;
 }
 
-}  // namespace iadmm
-
-using namespace iadmm;
-
-extern "C" {
-
-int iadmm_param_count(int h, int length, size_t* count) {
-  if (h <= 0 || length <= 0 || !count) IADMM_FAIL(IADMM_ESHAPE, "param_count: h=%d length=%d", h, length);
-  *count = grad_layout(h, length).total;
-  return IADMM_OK;
-}
-
-int iadmm_train_workspace_bytes(int B, int n, int m, int h, size_t* bytes) {
-  if (B <= 0 || n <= 0 || m < 0 || h <= 0 || !bytes) IADMM_FAIL(IADMM_ESHAPE, "train_workspace_bytes: B=%d n=%d m=%d h=%d", B, n, m, h);
-  TrainWs W;
-  plan_train(B, n, m, 0, h, nullptr, &W);
-  *bytes = W.bytes;
-  return IADMM_OK;
-}
-
-int iadmm_step_fwd(const void* packed_weights, const float* Q, const float* p, const float* A0, const float* zl,
-                   const float* zu, const float* x, const float* y, const float* z, const float* xv, const float* H,
-                   const float* C, float* x_o, float* y_o, float* z_o, float* xv_o, float* H_o, float* C_o,
-                   float* g_save, float* w_save, float* gates_save, int B, int n, int num_ineq, int num_eq, int h,
-                   int length, int t, float sigma, int mode, void* workspace, size_t workspace_bytes, void* stream) {
-  const int m = num_ineq + num_eq;
-  if (B <= 0 || n <= 0 || num_ineq < 0 || num_eq < 0 || h <= 0 || t < 0 || t >= length)
-    IADMM_FAIL(IADMM_ESHAPE, "step_fwd: B=%d n=%d ineq=%d eq=%d h=%d t=%d length=%d", B, n, num_ineq, num_eq, h, t, length);
-  if (B > 65535) IADMM_FAIL(IADMM_ESHAPE, "step_fwd: batch %d > 65535", B);
-  if (!packed_weights || !Q || !p || !x || !xv || !H || !C || !x_o || !xv_o || !H_o || !C_o || !g_save || !w_save || !workspace)
-    IADMM_FAIL(IADMM_EALIGN, "step_fwd: NULL pointer");            // gates_save may be NULL: activations not kept
-  if (h % 4 != 0) IADMM_FAIL(IADMM_ESHAPE, "step_fwd: hidden_dim %% 4 != 0 not supported by the training path");
-  int rc = check_device();
-  if (rc) return rc;
-  GatePlan gp;
-  if ((rc = plan_gates(mode, h, n, m, 1, 0, true, &gp))) return rc;
-  TrainWs W;
-  plan_train(B, n, m, num_ineq, h, workspace, &W);
-  if (W.bytes > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "step_fwd: workspace too small: %zu < %zu", workspace_bytes, W.bytes);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const WeightLayout L = weight_layout(h, length);
-  const char* wbase = static_cast<const char*>(packed_weights);
-  const Sched* sk = reinterpret_cast<const Sched*>(wbase + L.off_sched) + t;
-  const float* b_h = reinterpret_cast<const float*>(wbase + L.off_bh);
+// The body of iadmm_step_fwd at the width W.hp: weights `wimg` of layout L (L.h == W.hp), schedule row sk; H, C, H_o, C_o and
+// gates_save at that width.
+static int step_fwd_run(const void* wimg, const WeightLayout& L, const Sched* sk, const GatePlan& gp, const TrainWs& W,
+                        const float* Q, const float* p, const float* A0, const float* zl, const float* zu, const float* x,
+                        const float* y, const float* z, const float* xv, const float* H, const float* C, float* x_o, float* y_o,
+                        float* z_o, float* xv_o, float* H_o, float* C_o, float* g_save, float* w_save, float* gates_save, int B,
+                        int n, int m, float sigma, cudaStream_t st) {
+  const int h = W.hp;
+  const float* b_h = reinterpret_cast<const float*>(static_cast<const char*>(wimg) + L.off_bh);
   const size_t N = (size_t)n + m, rows = (size_t)B * N;
   const size_t fb = sizeof(float);
+  int rc;
   IADMM_CUDA(cudaMemcpyAsync(x_o, x, (size_t)B * n * fb, cudaMemcpyDeviceToDevice, st));
   if (m > 0) {
     IADMM_CUDA(cudaMemcpyAsync(y_o, y, (size_t)B * m * fb, cudaMemcpyDeviceToDevice, st));
@@ -572,42 +615,27 @@ int iadmm_step_fwd(const void* packed_weights, const float* Q, const float* p, c
   prof_end(kProfTrainKkt, st);
   // gate contraction of the forward: fp32 CUDA cores, or the tensor-core kernel (same arithmetic as the solve) with
   // the state converted at the boundary; both keep the gate activations for the backward
-  if ((rc = train_gate_forward(packed_weights, L, W, xv, W.s.g, H, H_o, C_o, gates_save, rows, h, gp, st))) return rc;
+  if ((rc = train_gate_forward(wimg, L, W, xv, W.s.g, H, H_o, C_o, gates_save, rows, h, gp, st))) return rc;
   return launch_tail(W.d, W.head_part, gp.head_slots, b_h, sk, zl, zu, x_o, y_o, z_o, xv_o, st);
 }
 
-int iadmm_step_bwd(const void* packed_weights, const float* Q, const float* p, const float* A0, const float* zl,
-                   const float* zu, const float* x, const float* y, const float* z, const float* xv, const float* H,
-                   const float* C, const float* xv_o, const float* H_o, const float* g_save, const float* w_save,
-                   const float* gates_save, const float* gx_o, const float* gy_o, const float* gz_o, const float* gxv_o,
-                   const float* gH_o, const float* gC_o, float* gx, float* gy, float* gz, float* gxv, float* gH, float* gC,
-                   float* grad_flat, int B, int n, int num_ineq, int num_eq, int h, int length, int t, float sigma,
-                   void* workspace, size_t workspace_bytes, void* stream) {
-  (void)p;
-  const int m = num_ineq + num_eq;
-  if (B <= 0 || n <= 0 || num_ineq < 0 || num_eq < 0 || h <= 0 || t < 0 || t >= length)
-    IADMM_FAIL(IADMM_ESHAPE, "step_bwd: B=%d n=%d ineq=%d eq=%d h=%d t=%d length=%d", B, n, num_ineq, num_eq, h, t, length);
-  if (!packed_weights || !Q || !x || !xv || !H || !C || !xv_o || !H_o || !g_save || !w_save || !gates_save || !gx || !gxv ||
-      !gH || !gC || !grad_flat || !workspace)
-    IADMM_FAIL(IADMM_EALIGN, "step_bwd: NULL pointer");
-  if (m > 0 && (!gy || !gz || !y || !z || !A0 || !zl || !zu)) IADMM_FAIL(IADMM_EALIGN, "step_bwd: NULL constraint pointer");
-  if (h % 4 != 0) IADMM_FAIL(IADMM_ESHAPE, "step_bwd: hidden_dim %% 4 != 0 not supported by the training path");
-  int rc = check_device();
-  if (rc) return rc;
-  TrainWs W;
-  plan_train(B, n, m, num_ineq, h, workspace, &W);
-  if (W.bytes > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "step_bwd: workspace too small: %zu < %zu", workspace_bytes, W.bytes);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const WeightLayout L = weight_layout(h, length);
-  const GradLayout G = grad_layout(h, length);
-  const char* wbase = static_cast<const char*>(packed_weights);
-  const Sched* sk = reinterpret_cast<const Sched*>(wbase + L.off_sched) + t;
+// The body of iadmm_step_bwd at the width W.hp (weights, state and adjoints as in step_fwd_run); the parameter adjoints are
+// added to grad_flat in the layout G of the caller's hidden_dim `hidden`, at schedule position t.
+static int step_bwd_run(const void* wimg, const WeightLayout& L, const Sched* sk, const TrainWs& W, int hidden, const GradLayout& G,
+                        int t, const float* Q, const float* A0, const float* zl, const float* zu, const float* x, const float* y,
+                        const float* z, const float* xv, const float* H, const float* C, const float* xv_o, const float* H_o,
+                        const float* g_save, const float* w_save, const float* gates_save, const float* gx_o, const float* gy_o,
+                        const float* gz_o, const float* gxv_o, const float* gH_o, const float* gC_o, float* gx, float* gy, float* gz,
+                        float* gxv, float* gH, float* gC, float* grad_flat, int B, int n, int m, float sigma, cudaStream_t st) {
+  const int h = W.hp;
+  const char* wbase = static_cast<const char*>(wimg);
   const float* u32 = reinterpret_cast<const float*>(wbase + L.off_u32);
   const float* wc = reinterpret_cast<const float*>(wbase + L.off_wc);
   const float* wh = reinterpret_cast<const float*>(wbase + L.off_wh);
   const size_t N = (size_t)n + m, rows = (size_t)B * N;
   const int h4 = 4 * h;
   const unsigned row_blocks = (unsigned)((rows + 255) / 256);
+  int rc;
 
   IADMM_CUDA(cudaMemsetAsync(W.zeros, 0, rows * sizeof(float), st));
   IADMM_CUDA(cudaMemsetAsync(W.zero_sched, 0, sizeof(Sched), st));
@@ -683,10 +711,118 @@ int iadmm_step_bwd(const void* packed_weights, const float* Q, const float* p, c
                                                     gxv, gx, gy, gz, W.acc);
   IADMM_LAUNCH_CHECK("step_bwd_final_kernel");
   // 8. parameters
-  scatter_grads_kernel<<<(unsigned)(((size_t)h * h4 + 255) / 256), 256, 0, st>>>(h, t, W.u32bar, W.w0bar, W.w1bar, W.bbar,
-                                                                                W.whbar, W.sbar_sum, W.acc, sk, G, grad_flat);
-  IADMM_LAUNCH_CHECK("scatter_grads_kernel");
+  if (hidden == h) {
+    scatter_grads_kernel<<<(unsigned)(((size_t)h * h4 + 255) / 256), 256, 0, st>>>(h, t, W.u32bar, W.w0bar, W.w1bar, W.bbar,
+                                                                                  W.whbar, W.sbar_sum, W.acc, sk, G, grad_flat);
+    IADMM_LAUNCH_CHECK("scatter_grads_kernel");
+  } else {
+    scatter_grads_padded_kernel<<<(unsigned)(((size_t)hidden * 4 * hidden + 255) / 256), 256, 0, st>>>(
+        hidden, h, t, W.u32bar, W.w0bar, W.w1bar, W.bbar, W.whbar, W.sbar_sum, W.acc, sk, G, grad_flat);
+    IADMM_LAUNCH_CHECK("scatter_grads_padded_kernel");
+  }
   return IADMM_OK;
+}
+
+static const Sched* sched_row(const void* wimg, const WeightLayout& L, int t) {
+  return reinterpret_cast<const Sched*>(static_cast<const char*>(wimg) + L.off_sched) + t;
+}
+
+}  // namespace iadmm
+
+using namespace iadmm;
+
+extern "C" {
+
+int iadmm_param_count(int h, int length, size_t* count) {
+  if (h <= 0 || length <= 0 || !count) IADMM_FAIL(IADMM_ESHAPE, "param_count: h=%d length=%d", h, length);
+  *count = grad_layout(h, length).total;
+  return IADMM_OK;
+}
+
+int iadmm_train_workspace_bytes(int B, int n, int m, int h, size_t* bytes) {
+  if (B <= 0 || n <= 0 || m < 0 || h <= 0 || !bytes) IADMM_FAIL(IADMM_ESHAPE, "train_workspace_bytes: B=%d n=%d m=%d h=%d", B, n, m, h);
+  TrainWs W;
+  plan_train(B, n, m, 0, h, true, nullptr, &W);
+  *bytes = W.bytes;
+  return IADMM_OK;
+}
+
+int iadmm_step_fwd(const void* packed_weights, const float* Q, const float* p, const float* A0, const float* zl,
+                   const float* zu, const float* x, const float* y, const float* z, const float* xv, const float* H,
+                   const float* C, float* x_o, float* y_o, float* z_o, float* xv_o, float* H_o, float* C_o,
+                   float* g_save, float* w_save, float* gates_save, int B, int n, int num_ineq, int num_eq, int h,
+                   int length, int t, float sigma, int mode, void* workspace, size_t workspace_bytes, void* stream) {
+  const int m = num_ineq + num_eq;
+  if (B <= 0 || n <= 0 || num_ineq < 0 || num_eq < 0 || h <= 0 || t < 0 || t >= length)
+    IADMM_FAIL(IADMM_ESHAPE, "step_fwd: B=%d n=%d ineq=%d eq=%d h=%d t=%d length=%d", B, n, num_ineq, num_eq, h, t, length);
+  if (B > 65535) IADMM_FAIL(IADMM_ESHAPE, "step_fwd: batch %d > 65535", B);
+  if (!packed_weights || !Q || !p || !x || !xv || !H || !C || !x_o || !xv_o || !H_o || !C_o || !g_save || !w_save || !workspace)
+    IADMM_FAIL(IADMM_EALIGN, "step_fwd: NULL pointer");            // gates_save may be NULL: activations not kept
+  int rc = check_device();
+  if (rc) return rc;
+  GatePlan gp;
+  if ((rc = plan_gates(mode, h, n, m, 1, 0, true, &gp))) return rc;
+  TrainWs W;
+  plan_train(B, n, m, num_ineq, h, true, workspace, &W);
+  if (W.bytes > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "step_fwd: workspace too small: %zu < %zu", workspace_bytes, W.bytes);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const WeightLayout L = weight_layout(h, length);
+  if (W.hp == h)
+    return step_fwd_run(packed_weights, L, sched_row(packed_weights, L, t), gp, W, Q, p, A0, zl, zu, x, y, z, xv, H, C, x_o, y_o,
+                        z_o, xv_o, H_o, C_o, g_save, w_save, gates_save, B, n, m, sigma, st);
+  // the zero-padded model of width hp: weights, state in, state out
+  const PadWs& P = W.pad;
+  const size_t rows = (size_t)B * (n + m);
+  if ((rc = pack_weights_padded(packed_weights, h, length, t, 1, W.hp, P.params, P.wimg, st))) return rc;
+  if ((rc = launch_repitch(H, h, P.H, W.hp, rows, st))) return rc;
+  if ((rc = launch_repitch(C, h, P.C, W.hp, rows, st))) return rc;
+  if ((rc = step_fwd_run(P.wimg, P.L, sched_row(P.wimg, P.L, 0), gp, W, Q, p, A0, zl, zu, x, y, z, xv, P.H, P.C, x_o, y_o, z_o,
+                         xv_o, P.H_o, P.C_o, g_save, w_save, gates_save, B, n, m, sigma, st))) return rc;
+  if ((rc = launch_repitch(P.H_o, W.hp, H_o, h, rows, st))) return rc;
+  return launch_repitch(P.C_o, W.hp, C_o, h, rows, st);
+}
+
+int iadmm_step_bwd(const void* packed_weights, const float* Q, const float* p, const float* A0, const float* zl,
+                   const float* zu, const float* x, const float* y, const float* z, const float* xv, const float* H,
+                   const float* C, const float* xv_o, const float* H_o, const float* g_save, const float* w_save,
+                   const float* gates_save, const float* gx_o, const float* gy_o, const float* gz_o, const float* gxv_o,
+                   const float* gH_o, const float* gC_o, float* gx, float* gy, float* gz, float* gxv, float* gH, float* gC,
+                   float* grad_flat, int B, int n, int num_ineq, int num_eq, int h, int length, int t, float sigma,
+                   void* workspace, size_t workspace_bytes, void* stream) {
+  (void)p;
+  const int m = num_ineq + num_eq;
+  if (B <= 0 || n <= 0 || num_ineq < 0 || num_eq < 0 || h <= 0 || t < 0 || t >= length)
+    IADMM_FAIL(IADMM_ESHAPE, "step_bwd: B=%d n=%d ineq=%d eq=%d h=%d t=%d length=%d", B, n, num_ineq, num_eq, h, t, length);
+  if (!packed_weights || !Q || !x || !xv || !H || !C || !xv_o || !H_o || !g_save || !w_save || !gates_save || !gx || !gxv ||
+      !gH || !gC || !grad_flat || !workspace)
+    IADMM_FAIL(IADMM_EALIGN, "step_bwd: NULL pointer");
+  if (m > 0 && (!gy || !gz || !y || !z || !A0 || !zl || !zu)) IADMM_FAIL(IADMM_EALIGN, "step_bwd: NULL constraint pointer");
+  int rc = check_device();
+  if (rc) return rc;
+  TrainWs W;
+  plan_train(B, n, m, num_ineq, h, true, workspace, &W);
+  if (W.bytes > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "step_bwd: workspace too small: %zu < %zu", workspace_bytes, W.bytes);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const WeightLayout L = weight_layout(h, length);
+  const GradLayout G = grad_layout(h, length);
+  const Sched* sk = sched_row(packed_weights, L, t);
+  if (W.hp == h)
+    return step_bwd_run(packed_weights, L, sk, W, h, G, t, Q, A0, zl, zu, x, y, z, xv, H, C, xv_o, H_o, g_save, w_save, gates_save,
+                        gx_o, gy_o, gz_o, gxv_o, gH_o, gC_o, gx, gy, gz, gxv, gH, gC, grad_flat, B, n, m, sigma, st);
+  // the zero-padded model of width hp (incoming adjoints that are NULL stay NULL = zero)
+  const PadWs& P = W.pad;
+  const size_t rows = (size_t)B * (n + m);
+  if ((rc = pack_weights_padded(packed_weights, h, length, t, 1, W.hp, P.params, P.wimg, st))) return rc;
+  if ((rc = launch_repitch(H, h, P.H, W.hp, rows, st))) return rc;
+  if ((rc = launch_repitch(C, h, P.C, W.hp, rows, st))) return rc;
+  if ((rc = launch_repitch(H_o, h, P.H_o, W.hp, rows, st))) return rc;
+  if (gH_o && (rc = launch_repitch(gH_o, h, P.gH_o, W.hp, rows, st))) return rc;
+  if (gC_o && (rc = launch_repitch(gC_o, h, P.gC_o, W.hp, rows, st))) return rc;
+  if ((rc = step_bwd_run(P.wimg, P.L, sched_row(P.wimg, P.L, 0), W, h, G, t, Q, A0, zl, zu, x, y, z, xv, P.H, P.C, xv_o, P.H_o,
+                         g_save, w_save, gates_save, gx_o, gy_o, gz_o, gxv_o, gH_o ? P.gH_o : nullptr, gC_o ? P.gC_o : nullptr,
+                         gx, gy, gz, gxv, P.gH, P.gC, grad_flat, B, n, m, sigma, st))) return rc;
+  if ((rc = launch_repitch(P.gH, W.hp, gH, h, rows, st))) return rc;
+  return launch_repitch(P.gC, W.hp, gC, h, rows, st);
 }
 
 // primal_dual_loss (utils.py:68-71) keeping the residual vectors for the backward
@@ -827,6 +963,8 @@ int iadmm_residuals_bwd(const float* Q, const float* A0, const float* pri, const
 namespace iadmm {
 
 struct WindowWs {
+  int hp;                                        // the width the kernels run at (train_hidden)
+  PadWs pad;                                     // hp != hidden_dim: the padded weights, schedule rows t0 .. t0+TL-1
   void* step_ws; size_t step_bytes;
   void* res_ws;  size_t res_bytes;
   float *x, *y, *z, *xv, *H, *C;                 // [TL+1] states each
@@ -837,14 +975,19 @@ struct WindowWs {
   size_t bytes;
 };
 
-static void plan_window(int B, int n, int m, int h, int TL, int flags, void* base, WindowWs* W) {
+// The window keeps its states and adjoints at the width hp = train_hidden(hidden): the caller's H and C are converted once on
+// entry and once on exit.
+static void plan_window(int B, int n, int m, int hidden, int TL, int flags, void* base, WindowWs* W) {
   const bool recompute = (flags & IADMM_TRAIN_RECOMPUTE_GATES) != 0;
   const size_t N = (size_t)n + m, rows = (size_t)B * N, fb = sizeof(float);
+  const int h = W->hp = train_hidden(hidden);
   char* p = static_cast<char*>(base);
   size_t off = 0;
+  W->pad = PadWs{};
+  if (h != hidden) plan_pad(hidden, TL, 0, p, &off, &W->pad);
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return base ? p + o : nullptr; };
   TrainWs T;
-  plan_train(B, n, m, 0, h, nullptr, &T);
+  plan_train(B, n, m, 0, hidden, false, nullptr, &T);
   W->step_bytes = T.bytes; W->step_ws = take(T.bytes);
   W->res_bytes = kkt_scratch_floats(make_kkt_dims_train(B, n, m, 0)) * fb + 1024; W->res_ws = take(W->res_bytes);
   const size_t S = (size_t)TL + 1;
@@ -936,16 +1079,32 @@ int iadmm_train_window(const void* packed_weights, const float* Q, const float* 
   if (!packed_weights || !Q || !p || !x || !xv || !H || !C || !grad_flat || !loss_out || !workspace)
     IADMM_FAIL(IADMM_EALIGN, "train_window: NULL pointer");
   if (m > 0 && (!A0 || !zl || !zu || !y || !z)) IADMM_FAIL(IADMM_EALIGN, "train_window: NULL constraint pointer");
+  if (B > 65535) IADMM_FAIL(IADMM_ESHAPE, "train_window: batch %d > 65535", B);
   GatePlan gp;
   int rc = plan_gates(mode, h, n, m, 1, 0, true, &gp);
   if (rc) return rc;
+  if ((rc = check_device())) return rc;
   const bool recompute = (flags & IADMM_TRAIN_RECOMPUTE_GATES) != 0;
   WindowWs W;
   plan_window(B, n, m, h, TL, flags, workspace, &W);
   if (W.bytes > workspace_bytes) IADMM_FAIL(IADMM_EWORK, "train_window: workspace too small: %zu < %zu", workspace_bytes, W.bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  TrainWs T;
+  plan_train(B, n, m, num_ineq, h, false, W.step_ws, &T);
+  if (T.bytes > W.step_bytes) IADMM_FAIL(IADMM_EWORK, "train_window: step workspace too small: %zu < %zu", W.step_bytes, T.bytes);
+  const int hp = W.hp;
   const size_t N = (size_t)n + m, rows = (size_t)B * N, fb = sizeof(float);
-  const size_t sx = (size_t)B * n, sy = (size_t)B * m, sxv = rows, sH = rows * h, sG = rows * 4 * h;
+  const size_t sx = (size_t)B * n, sy = (size_t)B * m, sxv = rows, sH = rows * hp, sG = rows * 4 * hp;
+  // the weights the kernels read, and the schedule row of iteration t0
+  const void* wimg = packed_weights;
+  WeightLayout Lw = weight_layout(h, length);
+  const Sched* sched0 = sched_row(wimg, Lw, t0);
+  if (hp != h) {
+    if ((rc = pack_weights_padded(packed_weights, h, length, t0, TL, hp, W.pad.params, W.pad.wimg, st))) return rc;
+    wimg = W.pad.wimg;
+    Lw = W.pad.L;
+    sched0 = sched_row(wimg, Lw, 0);
+  }
   // state 0 = the caller's state
   IADMM_CUDA(cudaMemcpyAsync(W.x, x, sx * fb, cudaMemcpyDeviceToDevice, st));
   if (m > 0) {
@@ -953,15 +1112,20 @@ int iadmm_train_window(const void* packed_weights, const float* Q, const float* 
     IADMM_CUDA(cudaMemcpyAsync(W.z, z, sy * fb, cudaMemcpyDeviceToDevice, st));
   }
   IADMM_CUDA(cudaMemcpyAsync(W.xv, xv, sxv * fb, cudaMemcpyDeviceToDevice, st));
-  IADMM_CUDA(cudaMemcpyAsync(W.H, H, sH * fb, cudaMemcpyDeviceToDevice, st));
-  IADMM_CUDA(cudaMemcpyAsync(W.C, C, sH * fb, cudaMemcpyDeviceToDevice, st));
+  if (hp == h) {
+    IADMM_CUDA(cudaMemcpyAsync(W.H, H, sH * fb, cudaMemcpyDeviceToDevice, st));
+    IADMM_CUDA(cudaMemcpyAsync(W.C, C, sH * fb, cudaMemcpyDeviceToDevice, st));
+  } else {
+    if ((rc = launch_repitch(H, h, W.H, hp, rows, st))) return rc;
+    if ((rc = launch_repitch(C, h, W.C, hp, rows, st))) return rc;
+  }
   // ---- forward sweep ----
   for (int t = 0; t < TL; ++t) {
     const size_t a = (size_t)t, b = (size_t)t + 1;
-    if ((rc = iadmm_step_fwd(packed_weights, Q, p, A0, zl, zu, W.x + a * sx, W.y + a * sy, W.z + a * sy, W.xv + a * sxv, W.H + a * sH,
-                             W.C + a * sH, W.x + b * sx, W.y + b * sy, W.z + b * sy, W.xv + b * sxv, W.H + b * sH, W.C + b * sH,
-                             W.g_save + a * sxv, W.w_save + a * sxv, recompute ? nullptr : W.gates + a * sG, B, n, num_ineq, num_eq, h,
-                             length, t0 + t, sigma, mode, W.step_ws, W.step_bytes, stream))) return rc;
+    if ((rc = step_fwd_run(wimg, Lw, sched0 + t, gp, T, Q, p, A0, zl, zu, W.x + a * sx, W.y + a * sy, W.z + a * sy, W.xv + a * sxv,
+                           W.H + a * sH, W.C + a * sH, W.x + b * sx, W.y + b * sy, W.z + b * sy, W.xv + b * sxv, W.H + b * sH,
+                           W.C + b * sH, W.g_save + a * sxv, W.w_save + a * sxv, recompute ? nullptr : W.gates + a * sG, B, n, m,
+                           sigma, st))) return rc;
     if ((rc = iadmm_residuals_fwd(W.x + b * sx, W.y + b * sy, W.z + b * sy, Q, p, A0, W.pri + a * B, W.dual + a * B, W.rp + a * sy,
                                   W.rd + a * sx, B, n, m, W.res_ws, W.res_bytes, stream))) return rc;
   }
@@ -994,19 +1158,16 @@ int iadmm_train_window(const void* packed_weights, const float* Q, const float* 
       // SURVEY section 7 step 6: the gate activations of iteration t are not kept over the window (25.6 MB per instance and
       // iteration at n+m = 2000, hidden_dim 800) but recomputed from the saved H_t, C_t, xv_t and g_t by the SAME kernel the
       // forward ran (bit-identical activations), into one iteration's worth of scratch
-      TrainWs T;
-      plan_train(B, n, m, num_ineq, h, W.step_ws, &T);
-      const WeightLayout Lw = weight_layout(h, length);
       IADMM_CUDA(cudaMemcpyAsync(W.Cs, W.C + a * sH, sH * fb, cudaMemcpyDeviceToDevice, st));
-      if ((rc = train_gate_forward(packed_weights, Lw, T, W.xv + a * sxv, W.g_save + a * sxv, W.H + a * sH, W.Hs, W.Cs, W.gates,
-                                   rows, h, gp, st))) return rc;
+      if ((rc = train_gate_forward(wimg, Lw, T, W.xv + a * sxv, W.g_save + a * sxv, W.H + a * sH, W.Hs, W.Cs, W.gates, rows, hp, gp,
+                                   st))) return rc;
       gates_t = W.gates;
     }
-    if ((rc = iadmm_step_bwd(packed_weights, Q, p, A0, zl, zu, W.x + a * sx, W.y + a * sy, W.z + a * sy, W.xv + a * sxv, W.H + a * sH,
-                             W.C + a * sH, W.xv + b * sxv, W.H + b * sH, W.g_save + a * sxv, W.w_save + a * sxv, gates_t,
-                             gin[0], m > 0 ? gin[1] : nullptr, m > 0 ? gin[2] : nullptr, last ? nullptr : gin[3],
-                             last ? nullptr : gin[4], last ? nullptr : gin[5], gout[0], gout[1], gout[2], gout[3], gout[4], gout[5],
-                             grad_flat, B, n, num_ineq, num_eq, h, length, t0 + t, sigma, W.step_ws, W.step_bytes, stream))) return rc;
+    if ((rc = step_bwd_run(wimg, Lw, sched0 + t, T, h, G, t0 + t, Q, A0, zl, zu, W.x + a * sx, W.y + a * sy, W.z + a * sy,
+                           W.xv + a * sxv, W.H + a * sH, W.C + a * sH, W.xv + b * sxv, W.H + b * sH, W.g_save + a * sxv,
+                           W.w_save + a * sxv, gates_t, gin[0], m > 0 ? gin[1] : nullptr, m > 0 ? gin[2] : nullptr,
+                           last ? nullptr : gin[3], last ? nullptr : gin[4], last ? nullptr : gin[5], gout[0], gout[1], gout[2],
+                           gout[3], gout[4], gout[5], grad_flat, B, n, m, sigma, st))) return rc;
     cur ^= 1;
   }
   // ---- the state leaving the window ----
@@ -1017,6 +1178,10 @@ int iadmm_train_window(const void* packed_weights, const float* Q, const float* 
     IADMM_CUDA(cudaMemcpyAsync(z, W.z + e * sy, sy * fb, cudaMemcpyDeviceToDevice, st));
   }
   IADMM_CUDA(cudaMemcpyAsync(xv, W.xv + e * sxv, sxv * fb, cudaMemcpyDeviceToDevice, st));
+  if (hp != h) {
+    if ((rc = launch_repitch(W.H + e * sH, hp, H, h, rows, st))) return rc;
+    return launch_repitch(W.C + e * sH, hp, C, h, rows, st);
+  }
   IADMM_CUDA(cudaMemcpyAsync(H, W.H + e * sH, sH * fb, cudaMemcpyDeviceToDevice, st));
   IADMM_CUDA(cudaMemcpyAsync(C, W.C + e * sH, sH * fb, cudaMemcpyDeviceToDevice, st));
   return IADMM_OK;

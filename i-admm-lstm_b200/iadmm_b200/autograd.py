@@ -45,7 +45,8 @@ class StepFunction(torch.autograd.Function):
         outs = [torch.empty_like(v) for v in (x, y, z, xv, H, C)]
         g_save = torch.empty((rows,), device=dev)
         w_save = torch.empty((rows,), device=dev)
-        gates = torch.empty((rows, 4 * h), device=dev)
+        hp = -(-h // 4) * 4            # the training kernels run hidden_dim rounded up to 4 (include/iadmm.h)
+        gates = torch.empty((rows, 4 * hp), device=dev)
         packed = model.packed_weights()
         ws = _train_ws(model, B, n, m, dev)
         with torch.cuda.device(dev):

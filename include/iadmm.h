@@ -253,12 +253,23 @@ int iadmm_lu_solve(const float* LU, const int* perm, float* rhs, int B, int N, v
  * iadmm_step_bwd (hand-written adjoint; reuses the two streaming KKT passes, two fp32 GEMMs for the gate
  * products).  The forward gate contraction runs in `mode` (IADMM_GATES_*, tensor cores by default like the solve;
  * F16F8 and F16F8U both keep the two correction products, as the 3-way split at hidden_dim % 16 == 8; a tensor-core mode
- * runs fp32 at hidden_dim % 8 != 0; an unknown mode is IADMM_EMODE); the backward is fp32 CUDA-core arithmetic.  Adam
- * (main.py:191) stays in PyTorch; data-parallel training all-reduces the flat gradient buffer over NCCL (iadmm_b200/dist.py).
+ * runs fp32 at hidden_dim % 8 != 0; an unknown mode is IADMM_EMODE); the backward's two gate-product GEMMs run on the
+ * tensor cores at hidden_dim % 16 == 0 and in fp32 on CUDA cores otherwise.  Adam (main.py:191) stays in PyTorch;
+ * data-parallel training all-reduces the flat gradient buffer over NCCL (iadmm_b200/dist.py).
+ *
+ * Every hidden_dim h >= 1 trains.  The kernels run the width hp = h rounded up to 4: for h % 4 != 0 each call re-lays the
+ * weights and the state into the model of width hp whose extra units have zero parameters and a zero state, and the results
+ * back.  Those units stay exactly zero (their gates are 0.5 and tanh(0)) and feed nothing into the real ones, so the outputs,
+ * adjoints and gradients are bit for bit those of the zero-padded width-hp model, and every rule above applies at hp: e.g.
+ * h = 50 runs the fp32 gates and backward of 52, h = 30 the tensor-core forward and backward of 32, h = 199 in tc_f16f8 the
+ * 3-way split of 200.  The caller-facing shapes stay at h (H, C and their adjoints [B*(n+m), h], grad_flat in the layout of
+ * iadmm_param_count(h, length), packed_weights the iadmm_pack_weights(h, length) image); the workspace-size queries include
+ * the padded copies.
  *
  * grad_flat: [iadmm_param_count] floats in state_dict order (W_i,U_i,b_i, W_f,.., W_u,U_u,b_u, W_h, b_h, rho,
  * alpha); iadmm_step_bwd ADDS this iteration's parameter adjoints to it.  Incoming adjoints g*_o may be
- * NULL (= zero); outgoing adjoints gx..gC are overwritten.  gates_save: [B*(n+m), 4h] (NULL in iadmm_step_fwd: not kept).
+ * NULL (= zero); outgoing adjoints gx..gC are overwritten.  gates_save: [B*(n+m), 4*hp] (NULL in iadmm_step_fwd: not kept),
+ * i.e. [B*(n+m), 4h] whenever h % 4 == 0.
  */
 int iadmm_param_count(int h, int length, size_t* count);
 int iadmm_train_workspace_bytes(int B, int n, int m, int h, size_t* bytes);
@@ -298,7 +309,7 @@ int iadmm_residuals_bwd(const float* Q, const float* A0, const float* pri, const
  * the state after the window (the reference detaches it there, main.py:353-358); grad_flat [iadmm_param_count] is
  * OVERWRITTEN with d loss / d parameters (state_dict order, see above); loss_out [1].  Same kernels and results as
  * the per-iteration entry points, without the host round trips between them. */
-enum { IADMM_TRAIN_RECOMPUTE_GATES = 1 };   /* flags of iadmm_train_window: do not keep the gate activations [TL, B*(n+m), 4h] over
+enum { IADMM_TRAIN_RECOMPUTE_GATES = 1 };   /* flags of iadmm_train_window: do not keep the gate activations [TL, B*(n+m), 4hp] over
                                                the window; the backward re-runs the forward gate kernel per iteration on the saved
                                                H, C, xv, g (bit-identical activations, same gradients): 2.56 -> 0 GB per instance
                                                and window at n+m = 2000, hidden_dim 800, TL = 100, for one more gate product */
